@@ -19,6 +19,11 @@ reports that variant beside the eager numbers under "cuda_graph" (single GPU, in
 
 --impl reference times the CPU restatement of the reference path (oracle/, all host threads) on the same
 workload, one batch item per step.  Prints ONE JSON line (rank 0).
+
+--dump-outputs DIR writes what the timed step returned in its last step (rank 0: the rendered maps rgb, seg, depth, wsum; the
+training step: its loss and the gradients it leaves on the planes and the decoder) as DIR/<name>.npy in float32.  The inputs are
+seeded, so two builds run with the same arguments can be compared output for output.  With N > 1 the training step's decoder
+gradients are rank 0's own: the step all-reduces a flattened copy of them and does not write the sum back.
 """
 import argparse
 import json
@@ -177,6 +182,36 @@ def make_inputs(torch, wl, device, seed):
     return raw_host, dec, c2w, k, opts
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """Write {name: tensor} as out_dir/<name>.npy in float32, at most `budget` bytes in all.  Arrays of up to 1 MB are stored
+    whole; when the larger ones do not fit in the rest of the budget, each keeps the same fraction of its rows (last dimension
+    whole; a vector's rows are its elements), picked with a fixed seed, so that two runs on the same shapes store the same
+    elements."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    header = 128                                    # bytes of a .npy header for these shapes
+    large = {n_ for n_, t in arrays.items() if t.numel() * 4 > (1 << 20)}
+    room = budget - sum(header + (0 if n_ in large else t.numel() * 4) for n_, t in arrays.items())
+    if room <= 0:
+        raise ValueError(f"the arrays of up to 1 MB alone fill the {budget}-byte budget")
+    total = sum(arrays[n_].numel() * 4 for n_ in large)
+    for name, t in arrays.items():
+        a = t.detach().float()
+        if name in large and total > room:
+            rows = a.reshape(-1, a.shape[-1] if a.dim() >= 2 else 1)
+            keep = rows.shape[0] * room // total
+            if keep == 0:                           # one row is wider than this array's share: sample elements instead
+                rows = a.reshape(-1, 1)
+                keep = rows.shape[0] * room // total
+            idx = np.sort(np.random.default_rng(0).choice(rows.shape[0], keep, replace=False))
+            a = rows[torch.from_numpy(idx).to(a.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+
+
 def hot_path_step(torch, mods, raw, dec, c2w, k, res, opts):
     """The public-API call sequence of TriPlaneGenerator.synthesis restricted to the hot path
     (triplane.py:84,95,113-119)."""
@@ -265,9 +300,14 @@ def main():
     ap.add_argument("--cuda-graph", action="store_true",
                     help="replay the step as ONE CUDA graph (nerffaceediting_b200.graphs; single-GPU inference workloads; "
                          "pays off where the step is launch-bound, i.e. c1)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed step returned in its last step to DIR/<name>.npy (float32; a fixed sample of rows when "
+                         f"the arrays exceed {DUMP_BYTES >> 20} MB)")
     args = ap.parse_args()
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
         return run_reference(args, wl)
 
     import torch
@@ -453,8 +493,9 @@ def main():
         launches0 = _lib.launch_count()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        last = fn()         # outside the loop, so that no step runs while the previous step's outputs are still held
         if sharded is not None:
             sharded.drain()                                       # the last steps' all-gathers are inside the timed region
         e1.record()
@@ -472,10 +513,10 @@ def main():
             t = torch.tensor([ms], device=device, dtype=torch.float64)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, launches, stages
+        return ms, launches, stages, last
 
     sampler = ClockSampler(local) if rank == 0 else None
-    ms_total, launches, stages = timed(step_resident, True)
+    ms_total, launches, stages, last = timed(step_resident, True)
     ms_eager = ms_total
     if args.cuda_graph:
         # the eager pass above supplies the per-stage events (they cannot be recorded inside a replay); the value is the replayed step
@@ -486,10 +527,19 @@ def main():
         graphed = {"resident": graphs.capture(lambda: hot_path_step(torch, mods, raw, dec, c2w, k, res, opts)),
                    "slot": [graphs.capture(lambda s_=s_: hot_path_step(torch, mods, dev_in[s_], dec, dev_cam[s_][0], dev_cam[s_][1], res, opts))
                             for s_ in (0, 1)]}
-        ms_total, _, _ = timed(step_resident, False)
+        ms_total, _, _, last = timed(step_resident, False)
         launches = graphed["resident"].kernels * steps
     clocks = sampler.stop() if sampler else None
-    ms_e2e, _, _ = timed(step_e2e, False)
+    if args.dump_outputs and rank == 0:
+        # before the e2e steps: they reset the gradients and (N > 1) reuse the gathered buffers
+        if train:
+            dumped = {"loss": last, "grad_planes": raw.grad, **{f"grad_decoder.{n_}": p_.grad for n_, p_ in dec.named_parameters()}}
+        else:
+            maps = last.wait() if world > 1 else last
+            dumped = {n_: t_ for n_, t_ in zip(("rgb", "seg", "depth", "wsum"), maps) if t_ is not None}
+        dump_outputs(args.dump_outputs, dumped)
+    del last
+    ms_e2e, _, _, _ = timed(step_e2e, False)
     h2d_gbs = None if train else h2d_rate_concurrent()
     graph_extra = None
     if not args.cuda_graph and not train and world == 1 and rays_per_rank * (wl["s_c"] + wl["s_f"]) <= (1 << 26):
@@ -497,7 +547,7 @@ def main():
         from nerffaceediting_b200 import graphs
         try:        # an extra beside the contract's numbers (all measured above): it must never cost the line
             graphed = {"resident": graphs.capture(lambda: hot_path_step(torch, mods, raw, dec, c2w, k, res, opts)), "slot": None}
-            ms_graph, _, _ = timed(step_resident, False)
+            ms_graph, _, _, _ = timed(step_resident, False)
             graph_extra = {"value": rays_per_rank / (ms_graph / steps * 1e-3), "unit": "rays/s", "ms_per_step": ms_graph / steps,
                            "kernels_per_replay": graphed["resident"].kernels,
                            "note": "same resident step captured once (nerffaceediting_b200.graphs.capture) and replayed with one launch per step; "
