@@ -15,7 +15,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "csrc", "_obj")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIB_DIR, "libnfe_b200.so")
-SOURCES = ["nfe_api.cu", "nfe_planes.cu", "nfe_rays.cu", "nfe_field.cu", "nfe_field_tc.cu", "nfe_field_pipe.cu", "nfe_field_pipe2.cu", "nfe_march.cu", "nfe_render.cu", "nfe_backward.cu", "nfe_field_bwd.cu", "nfe_diag.cu", "nfe_losses.cu", "nfe_stylegan_ops.cu", "nfe_modconv.cu"]
+SOURCES = ["nfe_api.cu", "nfe_planes.cu", "nfe_rays.cu", "nfe_field.cu", "nfe_field_tc.cu", "nfe_field_pipe2.cu", "nfe_march.cu", "nfe_render.cu", "nfe_backward.cu", "nfe_field_bwd.cu", "nfe_diag.cu", "nfe_losses.cu", "nfe_stylegan_ops.cu", "nfe_modconv.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC,-fvisibility=hidden", "--expt-relaxed-constexpr"]
 
@@ -33,7 +33,7 @@ def _newest_dep():
 
 def build(force=False, verbose=False):
     """Compile every .cu for sm_100a and link the shared library.  Returns the .so path.
-    $NFE_NVCC_FLAGS adds flags (e.g. -DNFE_GATHER_WARPS=8) for tuning sweeps on the GPU box."""
+    $NFE_NVCC_FLAGS adds flags (e.g. -DNFE_PIPE_PROFILE, the field kernel's role profiler) for experiments on the GPU box."""
     if not force and os.path.exists(LIB) and os.path.getmtime(LIB) >= _newest_dep():
         return LIB
     os.makedirs(OBJ, exist_ok=True)

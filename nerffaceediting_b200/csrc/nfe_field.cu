@@ -273,16 +273,7 @@ int launch_field(int kind, int precision, const FieldArgs& a, const nfe_mlp* net
     NFE_REQUIRE((int64_t)a.H * a.W * 3 * FEAT < (1ll << 31), "planes of %dx%d exceed the 32-bit texel offsets of the gather", a.H, a.W);
     NFE_REQUIRE((int64_t)a.plane_batch * a.H * a.W * 3 * (FEAT / 4) < (1ll << 31), "%d plane sets of %dx%d exceed the 32-bit texel offsets of the gather",
                 a.plane_batch, a.H, a.W);
-    if (precision != NFE_PREC_FP32) {
-        // NFE_TC_SIMPLE=1 selects the single-role tensor-core kernel (kept as the readable baseline of the pipelined one)
-        static const bool simple = getenv("NFE_TC_SIMPLE") != nullptr;
-        if (simple) return launch_field_tc(kind, precision, a, net_a, net_b, stream);
-        // NFE_FIELD_PIPE=1 selects round 1's kernel (4 epilogue warps, pre-pass inside the gather warps) for A/B runs
-        static const char* gen = getenv("NFE_FIELD_PIPE");
-        static const bool first_gen = gen && gen[0] == '1';
-        // (the experimental quad-order walk, NFE_QUAD_ORDER, only exists in round 1's kernel)
-        return (first_gen || a.quad_stride != 0) ? launch_field_pipe(kind, precision, a, net_a, net_b, stream) : launch_field_pipe2(kind, precision, a, net_a, net_b, stream);
-    }
+    if (precision != NFE_PREC_FP32) return launch_field_pipe2(kind, precision, a, net_a, net_b, stream);
     nfe_mlp none = {};
     switch (kind) {
         case NFE_DEC_OSG: return launch_field_kind<NFE_DEC_OSG>(a, *net_a, none, stream);
@@ -365,8 +356,7 @@ NFE_EXPORT int nfe_run_model_fwd(const nfe_render_cfg* cfg, const nfe_mlp* net_a
     const bool sigma_only = cfg->sigma_only != 0;
     const bool geo_only = sigma_only && cfg->kind == NFE_DEC_DISENTANGLED && cfg->precision != NFE_PREC_FP32;
     // single-gather identity (cfg->affine_*): the de-normalised planes are norm*scale + shift and are not read
-    const bool affine = cfg->affine_scale && cfg->affine_shift && cfg->kind == NFE_DEC_DISENTANGLED && cfg->precision != NFE_PREC_FP32 &&
-                        getenv("NFE_TC_SIMPLE") == nullptr;
+    const bool affine = cfg->affine_scale && cfg->affine_shift && cfg->kind == NFE_DEC_DISENTANGLED && cfg->precision != NFE_PREC_FP32;
     NFE_REQUIRE(!cfg->affine_scale || cfg->affine_items == 1 || cfg->affine_items == n, "nfe_run_model_fwd: affine statistics for %d items, batch is %d",
                 cfg->affine_items, n);
     NFE_REQUIRE((planes_denorm_cl || geo_only || affine) && coords && sigma && (rgb || sigma_only), "nfe_run_model_fwd: null pointer");

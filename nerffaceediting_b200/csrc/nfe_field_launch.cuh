@@ -22,12 +22,6 @@ struct FieldArgs {
     const float* dirs;
     const float* depths;      // [n*R*s_per_ray]
     int s_per_ray;
-    // Locality ordering (ray mode only; 0 = plain order): the rays of one batch item form a quad_stride x
-    // quad_stride image (ray m = row*quad_stride + col).  The pipelined kernel then walks samples as
-    // (4 vertically adjacent rays) x (depth index), so that the four samples of a gather pass share their
-    // (x,z)/(z,x)-plane texels and consecutive passes reuse the (x,y)-plane texels.
-    int quad_stride;
-    int64_t rays_per_item;
     int64_t m;                // samples per batch item
     int64_t total;            // n*m
     float* sigma;             // [total]
@@ -42,12 +36,10 @@ struct FieldArgs {
 };
 
 int check_decoder_dims(int kind, const nfe_mlp* net_a, const nfe_mlp* net_b, const char* who);
-// precision: NFE_PREC_FP32 -> SIMT fp32 kernel; NFE_PREC_BF16X3 / NFE_PREC_BF16 -> tcgen05 kernels (nfe_field_tc.cu)
+// precision: NFE_PREC_FP32 -> SIMT fp32 kernel (nfe_field.cu); NFE_PREC_BF16X3 / NFE_PREC_BF16 -> the tcgen05 kernel
+// (nfe_field_pipe2.cu)
 int launch_field(int kind, int precision, const FieldArgs& a, const nfe_mlp* net_a, const nfe_mlp* net_b, cudaStream_t stream);
-int launch_field_tc(int kind, int precision, const FieldArgs& a, const nfe_mlp* net_a, const nfe_mlp* net_b, cudaStream_t stream);
-// warp-specialised pipelined tensor-core kernel (nfe_field_pipe.cu): the production path for the tensor-core modes
-int launch_field_pipe(int kind, int precision, const FieldArgs& a, const nfe_mlp* net_a, const nfe_mlp* net_b, cudaStream_t stream);
-// second-generation pipelined kernel (nfe_field_pipe2.cu): two alternating epilogue groups, dedicated tap producers
+// warp-specialised pipelined tensor-core kernel: two alternating epilogue groups, dedicated tap producers
 int launch_field_pipe2(int kind, int precision, const FieldArgs& a, const nfe_mlp* net_a, const nfe_mlp* net_b, cudaStream_t stream);
 int launch_decoder_tc(int kind, int precision, const nfe_mlp* net_a, const nfe_mlp* net_b, const float* feat_norm, const float* feat_denorm,
                       int n, int64_t m, float* rgb, float* sigma, float* seg, cudaStream_t stream);

@@ -1,7 +1,8 @@
-// Field kernel, second generation: the same fused gather + decode on the tensor cores as nfe_field_pipe.cu, re-dealt so
-// that every SM sub-partition always has independent instruction streams to choose from (VERDICT r01 "next" #2).
+// Field kernel of the tensor-core precisions (bf16x3, bf16): fused gather + decode, warp-specialised so that every SM
+// sub-partition always has independent instruction streams to choose from (VERDICT r01 "next" #2).
 //
-// What round 1's kernel was bound by (profiles/ncu_r01_final_field_pipe_and_march.txt, profiles/l2_gather_r02.txt):
+// What round 1's kernel (4 epilogue warps, tap pre-pass inside the gather warps; since removed) was bound by
+// (profiles/ncu_r01_final_field_pipe_and_march.txt, profiles/l2_gather_r02.txt):
 //   * ONE epilogue warp per sub-partition ran a ~1500-instruction dependent chain per tile (softplus on the SFU, bf16 hi/lo
 //     split, TMEM traffic) at an IPC of 0.2 — 46 % of its stall samples were fixed-latency waits, nothing to overlap them with;
 //   * the 8 gather warps spent 30 % of their instructions in the tap pre-pass (position -> 12 offsets + 12 weights), run with
@@ -36,75 +37,37 @@ namespace p2 {
 
 constexpr int EPI_GROUPS = 2;
 constexpr int MMA_WARP = 8;
-#ifndef NFE_P2_TAP_WARPS
-#define NFE_P2_TAP_WARPS 3
-#endif
-constexpr int TAP_WARP0 = 9, TAP_WARPS = NFE_P2_TAP_WARPS;      // warps 9 .. 9 + TAP_WARPS - 1 (at most 3: warp 12 is the first gather warp)
+constexpr int TAP_WARP0 = 9, TAP_WARPS = 3;                 // warps 9 .. 9 + TAP_WARPS - 1 (at most 3: warp 12 is the first gather warp)
 static_assert(TAP_WARPS >= 1 && TAP_WARPS <= 3, "tap warps are warps 9-11");
-#ifndef NFE_P2_GATHER_WARPS
-#define NFE_P2_GATHER_WARPS 8
-#endif
-constexpr int GATHER_WARP0 = 12, GATHER_WARPS = NFE_P2_GATHER_WARPS;
+constexpr int GATHER_WARP0 = 12, GATHER_WARPS = 8;
 constexpr int THREADS = (GATHER_WARP0 + GATHER_WARPS) * 32;
 constexpr int PASSES_PER_TILE = TILE_M / 4;                 // a pass = 4 samples (8 lanes each)
 // consecutive passes of a tile each gather warp owns: the first LONG_WARPS warps take PER_LONG, the others PER_LONG - 1
-// (8 warps: 4 each; 12 warps: 8 x 3 + 4 x 2)
+// (8 warps: 4 each)
 constexpr int PER_LONG = (PASSES_PER_TILE + GATHER_WARPS - 1) / GATHER_WARPS;
 constexpr int LONG_WARPS = PASSES_PER_TILE - (PER_LONG - 1) * GATHER_WARPS;
 static_assert(LONG_WARPS >= 1 && LONG_WARPS <= GATHER_WARPS && PER_LONG >= 2, "bad gather split");
-#ifndef NFE_P2_TAP_BUFS
-#define NFE_P2_TAP_BUFS 3
-#endif
-constexpr int TAP_BUFS = NFE_P2_TAP_BUFS;                   // tap buffers: the tap warps run up to TAP_BUFS - 1 tiles ahead of the gather
+constexpr int TAP_BUFS = 3;                                 // tap buffers: the tap warps run up to TAP_BUFS - 1 tiles ahead of the gather
 constexpr int GROUP_COLS = 192;                             // D1A 64 | D1B 64 | D2A | D2B (<= 64 together)
 constexpr int P2_TMEM_COLS = 512;
 constexpr int COL_D2 = 128;
 constexpr int REC_STAGE_STRIDE = 208;                       // bytes per staged record row: conflict-free 16-byte stores
 
 // Register re-deal (setmaxnreg works on groups of four warps).  At launch every thread has what 640 threads allow (96).
-// Only registers a warp group RELEASES can be claimed by another (asking for more blocks forever), hence the static_assert.
+// Only registers a warp group RELEASES can be claimed by another (asking for more blocks forever), hence the static_asserts.
 // Measured at c2 (ms per launch, profiles/pipe2_variants_r02.txt): uniform 96: 0.355; epilogue/gather/misc = 104/104/64: 0.331
 // (the default); 96/112/56: 0.347; 104/112/48 and 112/104/48: 0.340-0.342 (at 48 the MMA-issuing thread spills and paces
 // everything); 12 gather warps at 80-88 registers: 0.445-0.57 (spills in the gather loop).
-#ifndef NFE_P2_SETMAXNREG
-#define NFE_P2_SETMAXNREG 1
-#endif
-#ifndef NFE_P2_REGS_EPI
-#define NFE_P2_REGS_EPI 104
-#endif
-#ifndef NFE_P2_REGS_MISC
-#define NFE_P2_REGS_MISC 64
-#endif
-#ifndef NFE_P2_UNROLL_PASSES
-#define NFE_P2_UNROLL_PASSES 0      // unrolling the passes of a tile trades loop bookkeeping for instruction-cache misses: slower
-#endif
-#ifndef NFE_P2_ROLLED_MMA
-#define NFE_P2_ROLLED_MMA 0
-#endif
-#ifndef NFE_P2_REGS_GATHER
-#define NFE_P2_REGS_GATHER 104
-#endif
-constexpr int REGS_LAUNCH = (65536 / THREADS) / 8 * 8 > 96 ? 96 : (65536 / THREADS) / 8 * 8;       // 20 warps: 96, 24 warps: 80
-constexpr int REGS_EPI = NFE_P2_REGS_EPI, REGS_MISC = NFE_P2_REGS_MISC, REGS_GATHER = NFE_P2_REGS_GATHER;
-static_assert(!NFE_P2_SETMAXNREG || (REGS_EPI >= REGS_LAUNCH && REGS_MISC <= REGS_LAUNCH), "epilogue groups only grow, the MMA / tap group only shrinks");
-static_assert(!NFE_P2_SETMAXNREG || (8 * (REGS_EPI - REGS_LAUNCH) + (REGS_GATHER > REGS_LAUNCH ? GATHER_WARPS * (REGS_GATHER - REGS_LAUNCH) : 0)
-                                     <= 4 * (REGS_LAUNCH - REGS_MISC) + (REGS_GATHER < REGS_LAUNCH ? GATHER_WARPS * (REGS_LAUNCH - REGS_GATHER) : 0)),
+constexpr int REGS_LAUNCH = 65536 / THREADS / 8 * 8;        // 96
+constexpr int REGS_EPI = 104, REGS_MISC = 64, REGS_GATHER = 104;
+static_assert(REGS_EPI > REGS_LAUNCH && REGS_GATHER > REGS_LAUNCH && REGS_MISC < REGS_LAUNCH,
+              "the epilogue and gather groups only grow, the MMA / tap group only shrinks");
+static_assert(8 * (REGS_EPI - REGS_LAUNCH) + GATHER_WARPS * (REGS_GATHER - REGS_LAUNCH) <= 4 * (REGS_LAUNCH - REGS_MISC),
               "setmaxnreg.inc would wait forever");
-static_assert(!NFE_P2_SETMAXNREG || (2 * REGS_EPI + REGS_MISC + (GATHER_WARPS / 4) * REGS_GATHER) * 32 <= 16384, "register file of a sub-partition");
+static_assert((2 * REGS_EPI + REGS_MISC + (GATHER_WARPS / 4) * REGS_GATHER) * 32 <= 16384, "register file of a sub-partition");
 
 constexpr float LOG2E = 1.4426950408889634f;
 constexpr float LN2 = 0.6931471805599453f;
-
-// NFE_P2_BIAS_MMA = 1: the layer-1 bias (and the log2(e) of the base-2 softplus) enter through the tensor core — log2(e) folded into W1,
-// the bias as one more K step whose A operand is a constant block of ones — so that the hidden epilogue neither reads the bias from
-// shared memory (13.8 % of the kernel's shared-memory wavefronts, the LSU being its busiest unit at 79 %) nor multiplies.  Parity green,
-// measured NEUTRAL (0.3040 vs 0.3042 ms per launch, profiles/pipe2_variants_r02.txt `bm*`): the epilogue groups only wait longer for
-// layer 2 (d2a_full 8.7 -> 15.5 %) — the gather warps pace the kernel — so the build keeps the plain epilogue.
-#ifndef NFE_P2_BIAS_MMA
-#define NFE_P2_BIAS_MMA 0
-#endif
-constexpr int ONES_LBO = 16 * 128, ONES_BYTES = 2 * ONES_LBO;            // [128 rows x 16]: column 0 = 1
-constexpr int BB_LBO = 8 * 128, BB_BYTES = 2 * BB_LBO;                   // [64 rows x 16]: column 0 = bias * log2(e)
 
 template <int KIND, bool SPLIT>
 struct Smem {
@@ -123,11 +86,9 @@ struct Smem {
     alignas(16) float aff[TAP_BUFS][2][2][96];          // [buffer][item - first item][scale | shift][channel]
     int aff_item[TAP_BUFS];
     alignas(16) unsigned char recbuf[EPI_GROUPS][TILE_M][REC_STAGE_STRIDE];   // record staging (each warp owns its 32 rows)
-    float bias1[NETS][HIDDEN];     // pre-multiplied by log2(e)
-#if NFE_P2_BIAS_MMA
-    alignas(128) unsigned char ones[ONES_BYTES];
-    alignas(128) unsigned char bias_op[NETS][PARTS][BB_BYTES];
-#endif
+    // layer-1 bias, pre-multiplied by log2(e).  Adding it through the tensor core instead (one more K step against a block of ones)
+    // measured neutral (profiles/pipe2_variants_r02.txt `bm*`): the gather warps pace the kernel, not the epilogue.
+    float bias1[NETS][HIDDEN];
     float bias2a[T::N_A];
     float bias2b[T::N_B];
     alignas(8) uint64_t full[2], empty[2];                                // feature ring
@@ -147,30 +108,13 @@ __device__ void load_params(Smem<KIND, SPLIT>& s, const nfe_mlp& net_a, const nf
 {
     using T = TcTraits<KIND>;
     constexpr int PARTS = SPLIT ? 2 : 1;
-    constexpr float W1_FOLD = NFE_P2_BIAS_MMA ? LOG2E : 1.0f;
-    constexpr int NETS = T::HAS_B ? 2 : 1;
-    (void)NETS;
-    load_weights<PARTS>(s.b1[0][0], B1_BYTES, net_a.w1, net_a.wgain1 * W1_FOLD, HIDDEN, HIDDEN, FEAT, B1_LBO, B1_SBO);
-#if NFE_P2_BIAS_MMA
-    for (int i = threadIdx.x; i < ONES_BYTES / 2; i += blockDim.x) {                 // element (row, k) of the ones block
-        const int row = (i >> 3) & 127, k = (i & 7) + 8 * (i >> 10);
-        *reinterpret_cast<__nv_bfloat16*>(s.ones + core_offset(row, k, ONES_LBO, 128)) = __float2bfloat16_rn(k == 0 ? 1.0f : 0.0f);
-    }
-    for (int i = threadIdx.x; i < NETS * HIDDEN * 16; i += blockDim.x) {
-        const int net = i / (HIDDEN * 16), n = (i / 16) % HIDDEN, k = i % 16;
-        const nfe_mlp& m = net ? net_b : net_a;
-        __nv_bfloat16 hi, lo;
-        tc::split_bf16(k == 0 ? folded_bias(m.b1, m.bgain1, n) * LOG2E : 0.0f, hi, lo);
-        *reinterpret_cast<__nv_bfloat16*>(s.bias_op[net][0] + core_offset(n, k, BB_LBO, 128)) = hi;
-        if (PARTS == 2) *reinterpret_cast<__nv_bfloat16*>(s.bias_op[net][PARTS - 1] + core_offset(n, k, BB_LBO, 128)) = lo;
-    }
-#endif
+    load_weights<PARTS>(s.b1[0][0], B1_BYTES, net_a.w1, net_a.wgain1, HIDDEN, HIDDEN, FEAT, B1_LBO, B1_SBO);
     // softplus runs in base 2 (see hidden_in_place): ln 2 goes into the layer-2 weights, log2(e) into the layer-1 bias
     load_weights<PARTS>(s.b2a[0], sizeof(s.b2a[0]), net_a.w2, net_a.wgain2 * LN2, T::OUT_A, T::N_A, HIDDEN, B2_LBO, B2_SBO);
     for (int i = threadIdx.x; i < HIDDEN; i += blockDim.x) s.bias1[0][i] = folded_bias(net_a.b1, net_a.bgain1, i) * LOG2E;
     for (int i = threadIdx.x; i < T::N_A; i += blockDim.x) s.bias2a[i] = i < T::OUT_A ? folded_bias(net_a.b2, net_a.bgain2, i) : 0.0f;
     if constexpr (T::HAS_B) {
-        load_weights<PARTS>(s.b1[1][0], B1_BYTES, net_b.w1, net_b.wgain1 * W1_FOLD, HIDDEN, HIDDEN, FEAT, B1_LBO, B1_SBO);
+        load_weights<PARTS>(s.b1[1][0], B1_BYTES, net_b.w1, net_b.wgain1, HIDDEN, HIDDEN, FEAT, B1_LBO, B1_SBO);
         load_weights<PARTS>(s.b2b[0], sizeof(s.b2b[0]), net_b.w2, net_b.wgain2 * LN2, T::OUT_B, T::N_B, HIDDEN, B2_LBO, B2_SBO);
         for (int i = threadIdx.x; i < HIDDEN; i += blockDim.x) s.bias1[1][i] = folded_bias(net_b.b1, net_b.bgain1, i) * LOG2E;
         for (int i = threadIdx.x; i < T::N_B; i += blockDim.x) s.bias2b[i] = i < T::OUT_B ? folded_bias(net_b.b2, net_b.bgain2, i) : 0.0f;
@@ -193,15 +137,12 @@ __device__ __forceinline__ float2 rgb_activation2(float2 x)
 // hidden = softplus(D1 + b1) for this thread's row, written back over the accumulator columns it came from: the 16 fp32
 // columns [16q, 16q+16) become 8 columns of packed bf16 hi parts at 16q and 8 columns of lo parts at 16q+8.
 // Softplus in base-2 units: with t = x*log2(e), softplus(x) = ln2 * (max(t,0) + log2(1 + 2^-|t|)).
-#ifndef NFE_P2_HIDDEN_UNROLL
-#define NFE_P2_HIDDEN_UNROLL 1      // copies of the 16-column body in the loop (1: smallest code; the kernel is instruction-cache sensitive)
-#endif
-constexpr int HIDDEN_UNROLL = NFE_P2_HIDDEN_UNROLL;
 template <bool SPLIT>
 __device__ __forceinline__ void hidden_in_place(uint32_t taddr, const float* bias1_log2)
 {
     const float2 k2 = make_float2(LOG2E, LOG2E), one2 = make_float2(1.0f, 1.0f), neg2 = make_float2(-1.0f, -1.0f);
-#pragma unroll HIDDEN_UNROLL
+    // one copy of the 16-column body: smallest code, and the kernel is instruction-cache sensitive
+#pragma unroll 1
     for (int q = 0; q < HIDDEN / 16; ++q) {
         float v[16];
         tc::tmem_ld16(taddr + q * 16, v);
@@ -209,16 +150,10 @@ __device__ __forceinline__ void hidden_in_place(uint32_t taddr, const float* bia
         uint32_t hi[8], lo[8];
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
-#if !NFE_P2_BIAS_MMA
             const float4 b4 = *reinterpret_cast<const float4*>(bias1_log2 + q * 16 + 4 * i);
-#endif
 #pragma unroll
             for (int j = 0; j < 2; ++j) {
-#if NFE_P2_BIAS_MMA
-                const float2 t = make_float2(v[4 * i + 2 * j], v[4 * i + 2 * j + 1]);            // the accumulator already is (x W1^T + b1) * log2(e)
-#else
                 const float2 t = ffma2(make_float2(v[4 * i + 2 * j], v[4 * i + 2 * j + 1]), k2, j ? make_float2(b4.z, b4.w) : make_float2(b4.x, b4.y));
-#endif
                 float e0, e1, l0, l1;
                 asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e0) : "f"(-fabsf(t.x)));
                 asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e1) : "f"(-fabsf(t.y)));
@@ -250,19 +185,11 @@ __device__ __forceinline__ void issue_layer2(bool leader, uint32_t tmem_d, uint3
     const uint64_t db0 = tc::make_desc(0, B2_LBO, B2_SBO);
     const uint32_t bh = tc::smem_u32(b_hi) >> 4, bl = tc::smem_u32(b_lo) >> 4;
     constexpr int TERMS = SPLIT ? 3 : 1;
-#if NFE_P2_ROLLED_MMA
-#pragma unroll 1
-#else
 #pragma unroll
-#endif
     for (int t = 0; t < TERMS; ++t) {
         const uint32_t part = (t == 1) ? 8u : 0u;                        // hi*hi, lo*hi, hi*lo
         const uint32_t b = (t == 2) ? bl : bh;
-#if NFE_P2_ROLLED_MMA
-#pragma unroll 1
-#else
 #pragma unroll
-#endif
         for (int ks = 0; ks < HIDDEN / 16; ++ks) {
             if (leader) tc::mma_bf16_ts(tmem_d, tmem_h + ks * 16 + part, db0 + (b + ks * ((2 * B2_LBO) >> 4)), idesc, acc);
             acc = 1;
@@ -272,7 +199,7 @@ __device__ __forceinline__ void issue_layer2(bool leader, uint32_t tmem_d, uint3
 
 struct SampleRef { int64_t idx; int item; int64_t ray; };
 
-// Tile row -> sample.  Plain order only: sample L is index L (the quad-order walk of FieldArgs::quad_stride stays with round 1's kernel)
+// Tile row -> sample: sample L is index L, in batch item L / m, on ray L / s_per_ray
 __device__ __forceinline__ SampleRef sample_of(const FieldArgs& a, int64_t L, bool small)
 {
     SampleRef r;
@@ -287,16 +214,13 @@ __device__ __forceinline__ SampleRef sample_of(const FieldArgs& a, int64_t L, bo
     return r;
 }
 
-#ifndef NFE_TAP_CG
-#define NFE_TAP_CG 1
-#endif
 // texel load at lane_base + 16*off4 (one IMAD.WIDE + LDG); `streaming` taps (planes 1 and 2: no reuse between the samples a
 // warp walks) bypass L1 allocation, plane 0 keeps the read-only path where consecutive samples of a ray share texels
 __device__ __forceinline__ float4 ldg_tap(const float4* lane_base, uint32_t off4, bool streaming)
 {
     uint64_t addr;
     asm("mad.wide.u32 %0, %1, 16, %2;" : "=l"(addr) : "r"(off4), "l"(lane_base));
-    if (NFE_TAP_CG == 2 || (NFE_TAP_CG == 1 && streaming)) return __ldcg(reinterpret_cast<const float4*>(addr));
+    if (streaming) return __ldcg(reinterpret_cast<const float4*>(addr));
     return __ldg(reinterpret_cast<const float4*>(addr));
 }
 
@@ -377,10 +301,7 @@ __global__ void __launch_bounds__(THREADS, 1) field_pipe2_kernel(FieldArgs a, nf
         const int n_pass = gw < LONG_WARPS ? PER_LONG : PER_LONG - 1;
         const int pass0 = gw < LONG_WARPS ? gw * PER_LONG : LONG_WARPS * PER_LONG + (gw - LONG_WARPS) * (PER_LONG - 1);
         const int row0 = 4 * pass0 + g;                     // this lane group's row in its first pass of a tile; pass p: + 4p
-#if NFE_P2_SETMAXNREG
-        if (REGS_GATHER > REGS_LAUNCH) regs_inc<REGS_GATHER>();
-        else if (REGS_GATHER < REGS_LAUNCH) regs_dec<REGS_GATHER>();
-#endif
+        regs_inc<REGS_GATHER>();
 
         float4 va[12];                    // rolling pipeline: the texels of the NEXT pass, in flight while this one is blended
         if (n_my > 0) {
@@ -401,16 +322,12 @@ __global__ void __launch_bounds__(THREADS, 1) field_pipe2_kernel(FieldArgs a, nf
             const bool has_next = it + 1 < n_my;
             P2_WAIT(1, &s.empty[st], ((it >> 1) & 1) ^ 1);      // slot released by the layer-1 commit two tiles ago
             if (rolling) {
-                // the passes of a tile are unrolled (shared-memory addresses become base + constant, no loop bookkeeping): the
-                // body is instantiated for the two pass counts a warp can own
+                // the body is instantiated for the two pass counts a warp can own; the pass loop stays rolled: unrolling it
+                // trades loop bookkeeping for instruction-cache misses, which measured slower
                 auto tile_body = [&](auto np_tag) {
                     constexpr int NP = decltype(np_tag)::value;
                     const uint4* tap_row = s.taps[tb][row0];
-#if NFE_P2_UNROLL_PASSES
-#pragma unroll
-#else
 #pragma unroll 1
-#endif
                     for (int p = 0; p < NP; ++p) {
                         const int row = row0 + 4 * p;
                         const uint4* cur = tap_row + 4 * p * 7;
@@ -500,9 +417,7 @@ __global__ void __launch_bounds__(THREADS, 1) field_pipe2_kernel(FieldArgs a, nf
         // ONE lane per sample turns its position into 12 clamped texel offsets + 12 weights (zero for taps that fall
         // outside: padding_mode='zeros') and parks them in shared memory for the 8 gather lanes of that sample.
         const int tw = warp - TAP_WARP0;
-#if NFE_P2_SETMAXNREG
         regs_dec<REGS_MISC>();
-#endif
         const int64_t set_stride4 = (int64_t)3 * a.H * a.W * (FEAT / 4);     // float4 units
         const bool small = a.total < (1ll << 31);
         // row-wise deal: every tap warp works on every tile — the four 32-sample chunks of a tile go to warps 0 .. TAP_WARPS-1, the
@@ -610,9 +525,7 @@ __global__ void __launch_bounds__(THREADS, 1) field_pipe2_kernel(FieldArgs a, nf
     } else if (warp == MMA_WARP) {
         // ================================================================ MMA issuer: every lane runs the (warp-uniform) loop, one
         // elected lane issues — see tc::elect_one
-#if NFE_P2_SETMAXNREG
         regs_dec<REGS_MISC>();
-#endif
         {
             const bool leader = tc::elect_one();
             constexpr uint32_t idesc1 = tc::make_idesc_bf16(TILE_M, HIDDEN);
@@ -625,20 +538,9 @@ __global__ void __launch_bounds__(THREADS, 1) field_pipe2_kernel(FieldArgs a, nf
                 P2_WAIT(3, &s.full[st], (it >> 1) & 1);          // features landed
                 tc::fence_after_sync();
                 issue_gemm<SPLIT>(leader, tb + COL_D1A, s.a1[st][0][0], s.a1[st][0][P], A1_LBO, A1_SBO, s.b1[0][0], s.b1[0][P], B1_LBO, B1_SBO, FEAT, idesc1);
-#if NFE_P2_BIAS_MMA
-                auto bias_step = [&](uint32_t d, int net) {                 // D += ones * (bias_hi + bias_lo)^T, one K = 16 step each
-                    const uint64_t da = tc::make_desc(tc::smem_u32(s.ones), ONES_LBO, 128);
-                    if (leader) tc::mma_bf16_ss(d, da, tc::make_desc(tc::smem_u32(s.bias_op[net][0]), BB_LBO, 128), idesc1, 1);
-                    if (SPLIT && leader) tc::mma_bf16_ss(d, da, tc::make_desc(tc::smem_u32(s.bias_op[net][P]), BB_LBO, 128), idesc1, 1);
-                };
-                bias_step(tb + COL_D1A, 0);
-#endif
                 if (has_b)
                     issue_gemm<SPLIT>(leader, tb + COL_D1B, s.a1[st][T::SETS - 1][0], s.a1[st][T::SETS - 1][P], A1_LBO, A1_SBO, s.b1[T::HAS_B ? 1 : 0][0],
                                       s.b1[T::HAS_B ? 1 : 0][P], B1_LBO, B1_SBO, FEAT, idesc1);
-#if NFE_P2_BIAS_MMA
-                if (has_b) bias_step(tb + COL_D1B, T::HAS_B ? 1 : 0);
-#endif
                 if (leader) {
                     tc::mma_commit(&s.empty[st]);                   // ring slot reusable once these MMAs have read it
                     tc::mma_commit(&s.d1_full[st]);
@@ -674,9 +576,7 @@ __global__ void __launch_bounds__(THREADS, 1) field_pipe2_kernel(FieldArgs a, nf
     } else if (warp < MMA_WARP) {
         // ================================================================ epilogue groups (TMEM lanes 32*(warp&3) ..)
         const int gi = warp >> 2, wq = warp & 3;
-#if NFE_P2_SETMAXNREG
-        if (REGS_EPI > REGS_LAUNCH) regs_inc<REGS_EPI>();
-#endif
+        regs_inc<REGS_EPI>();
         const int row = wq * 32 + lane;
         const uint32_t lane_addr = tmem + gi * GROUP_COLS + ((uint32_t)(wq * 32) << 16);
         uint32_t ph = 0;
@@ -836,13 +736,9 @@ __global__ void __launch_bounds__(THREADS, 1) field_pipe2_kernel(FieldArgs a, nf
                 __syncwarp();          // the rows are rewritten by the group's next tile
             }
         }
-    }
-
-#if NFE_P2_SETMAXNREG
-    else {
+    } else {
         regs_dec<REGS_MISC>();            // idle warps of the MMA / tap warp group: setmaxnreg is a warp-group-wide instruction
     }
-#endif
 #ifdef NFE_PIPE_PROFILE
     if (lane == 0 && !(warp > TAP_WARP0 + TAP_WARPS - 1 && warp < GATHER_WARP0)) {
         const int role = warp >= GATHER_WARP0 ? 0 : (warp >= TAP_WARP0 ? 1 : (warp == MMA_WARP ? 2 : 3));

@@ -1,5 +1,5 @@
-// Tensor-core (tcgen05 + TMEM) variants of the decoder and of the fused gather+decode kernel.
-// See nfe_mlp_tc.cuh for the GEMM formulation; this file owns the CTA-level choreography:
+// Tensor-core (tcgen05 + TMEM) path of the stand-alone decoder (nfe_decoder_fwd in the bf16x3 / bf16 precisions) on
+// materialised features.  See nfe_mlp_tc.cuh for the GEMM formulation; this file owns the CTA-level choreography:
 //
 //   all threads   build the 128-row feature tile (bf16 hi/lo parts) in shared memory
 //   fence.proxy.async + barrier
@@ -130,123 +130,6 @@ __global__ void __launch_bounds__(TILE_M, 1) decoder_tc_kernel(nfe_mlp net_a, nf
         tc::fence_after_sync();
     }
     tc_teardown(s);
-}
-
-// ------------------------------------------------------------------------------------------
-// Fused gather + decode on the tensor cores.  A CTA step covers 128 consecutive samples:
-// warp w gathers rows 32w..32w+31 (8 passes of 4 samples, 8 lanes per sample, as the fp32 kernel)
-// straight into the bf16 feature tile, then the four warps become the TMEM epilogue.
-// ------------------------------------------------------------------------------------------
-template <int KIND, bool SPLIT>
-__global__ void __launch_bounds__(TILE_M, 1) field_tc_kernel(FieldArgs a, nfe_mlp net_a, nfe_mlp net_b)
-{
-    using T = TcTraits<KIND>;
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    Smem<KIND, SPLIT>& s = *reinterpret_cast<Smem<KIND, SPLIT>*>(smem_raw);
-    tc_setup(s, net_a, net_b);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int g = lane >> 3, c4 = lane & 7;
-    const int64_t set_stride = (int64_t)3 * a.H * a.W * FEAT;
-    const int64_t n_tiles = (a.total + TILE_M - 1) / TILE_M;
-    uint32_t parity = 0;
-    for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, parity ^= 1) {
-        const int64_t base = tile * TILE_M;
-#pragma unroll 2
-        for (int j = 0; j < 8; ++j) {
-            const int row = warp * 32 + 4 * j + g;
-            const int64_t idx = base + row;
-            float4 fa = make_float4(0.f, 0.f, 0.f, 0.f), fb = fa;
-            if (idx < a.total) {
-                float x, y, z;
-                if (a.coords) {
-                    const float* c = a.coords + idx * 3;
-                    x = __ldg(c); y = __ldg(c + 1); z = __ldg(c + 2);
-                } else {
-                    const int64_t ray = idx / a.s_per_ray;
-                    const float t = __ldg(a.depths + idx);
-                    const float* o = a.origins + ray * 3;
-                    const float* d = a.dirs + ray * 3;
-                    x = ray_point(__ldg(o), t, __ldg(d)); y = ray_point(__ldg(o + 1), t, __ldg(d + 1)); z = ray_point(__ldg(o + 2), t, __ldg(d + 2));
-                }
-                const int64_t pbi = a.plane_batch == 1 ? 0 : idx / a.m;
-                const TapSet ts = make_tapset(taps3(__fmul_rn(a.scale, x), __fmul_rn(a.scale, y), __fmul_rn(a.scale, z), a.H, a.W), a.H, a.W);
-                float4 va[12], vb[12];
-                if (T::SETS == 2) gather_load(a.set_norm + pbi * set_stride, ts, c4, va);
-                gather_load(a.set_denorm + pbi * set_stride, ts, c4, vb);
-                if (T::SETS == 2) fa = gather_reduce(va, ts);
-                fb = gather_reduce(vb, ts);
-            }
-            if (T::SETS == 2) store_features4<SPLIT>(s.a1[0], row, 4 * c4, fa);
-            store_features4<SPLIT>(s.a1[T::SETS - 1], row, 4 * c4, fb);
-        }
-        float sig, segv[16], col[32];
-        tc_decode_tile<KIND, SPLIT>(s, parity, sig, segv, col);
-        const int64_t idx = base + threadIdx.x;
-        if (idx < a.total) {
-            if (a.density_noise > 0.0f) {
-                const uint4 r = philox4x32(a.seed, (uint64_t)idx, a.offset);
-                sig += normal2(r.x, r.y).x * a.density_noise;
-            }
-            a.sigma[idx] = sig;
-            if (a.sigma_only) goto next_tile;
-            float4* rec = a.rec ? reinterpret_cast<float4*>(a.rec + idx * 48) : nullptr;
-            float4* rgb4 = rec ? rec + 4 : reinterpret_cast<float4*>(a.rgb + idx * 32);
-#pragma unroll
-            for (int c = 0; c < 8; ++c) rgb4[c] = make_float4(col[4 * c], col[4 * c + 1], col[4 * c + 2], col[4 * c + 3]);
-            if (rec) {
-                if (!T::HAS_B) {
-#pragma unroll
-                    for (int c = 0; c < 15; ++c) segv[c] = 0.0f;
-                }
-                rec[0] = make_float4(sig, segv[0], segv[1], segv[2]);
-#pragma unroll
-                for (int c = 1; c < 4; ++c) rec[c] = make_float4(segv[4 * c - 1], segv[4 * c], segv[4 * c + 1], segv[4 * c + 2]);
-            } else if constexpr (T::HAS_B) {
-#pragma unroll
-                for (int c = 0; c < 15; ++c) a.seg[idx * 15 + c] = segv[c];
-            }
-        }
-    next_tile:
-        tc::fence_before_sync();
-        __syncthreads();
-        tc::fence_after_sync();
-    }
-    tc_teardown(s);
-}
-
-template <int KIND, bool SPLIT>
-static int launch_field_tc_kind(const FieldArgs& a, const nfe_mlp& net_a, const nfe_mlp& net_b, cudaStream_t stream)
-{
-    const size_t smem = sizeof(Smem<KIND, SPLIT>) + 128;
-    static bool configured = false;
-    if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(field_tc_kernel<KIND, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) { set_error("field_tc_kernel: cannot reserve %zu bytes of shared memory: %s", smem, cudaGetErrorString(e)); return 2; }
-        configured = true;
-    }
-    const int64_t n_tiles = (a.total + TILE_M - 1) / TILE_M;
-    // TMEM: 256 columns per CTA -> at most 2 CTAs per SM
-    const int64_t cap = (int64_t)sm_count() * (smem <= 110 * 1024 ? 2 : 1);
-    field_tc_kernel<KIND, SPLIT><<<(unsigned)(n_tiles < cap ? n_tiles : cap), TILE_M, smem, stream>>>(a, net_a, net_b);
-    return check_launch("field_tc_kernel");
-}
-
-int launch_field_tc(int kind, int precision, const FieldArgs& a, const nfe_mlp* net_a, const nfe_mlp* net_b, cudaStream_t stream)
-{
-    if (a.total <= 0) return 0;
-    nfe_mlp none = {};
-    const bool split = precision == NFE_PREC_BF16X3;
-    switch (kind) {
-        case NFE_DEC_OSG:
-            return split ? launch_field_tc_kind<NFE_DEC_OSG, true>(a, *net_a, none, stream) : launch_field_tc_kind<NFE_DEC_OSG, false>(a, *net_a, none, stream);
-        case NFE_DEC_DISENTANGLED:
-            return split ? launch_field_tc_kind<NFE_DEC_DISENTANGLED, true>(a, *net_a, *net_b, stream)
-                         : launch_field_tc_kind<NFE_DEC_DISENTANGLED, false>(a, *net_a, *net_b, stream);
-        default:
-            return split ? launch_field_tc_kind<NFE_DEC_SEGMENTATION, true>(a, *net_a, *net_b, stream)
-                         : launch_field_tc_kind<NFE_DEC_SEGMENTATION, false>(a, *net_a, *net_b, stream);
-    }
 }
 
 template <int KIND, bool SPLIT>

@@ -86,8 +86,7 @@ NFE_EXPORT int nfe_render_fwd(const nfe_render_cfg* cfg, const nfe_mlp* net_a, c
     if (int rc = check_cfg(cfg, "nfe_render_fwd")) return rc;
     if (int rc = check_decoder_dims(cfg->kind, net_a, net_b, "nfe_render_fwd")) return rc;
     if ((int64_t)n * n_rays == 0) return 0;  // empty tensors carry null pointers
-    static const bool tc_simple = getenv("NFE_TC_SIMPLE") != nullptr;
-    const bool affine = cfg->affine_scale && cfg->affine_shift && cfg->kind == NFE_DEC_DISENTANGLED && cfg->precision != NFE_PREC_FP32 && !tc_simple;
+    const bool affine = cfg->affine_scale && cfg->affine_shift && cfg->kind == NFE_DEC_DISENTANGLED && cfg->precision != NFE_PREC_FP32;
     NFE_REQUIRE(!cfg->affine_scale || (cfg->affine_items == 1 || cfg->affine_items == n), "nfe_render_fwd: affine statistics for %d items, batch is %d",
                 cfg->affine_items, n);
     NFE_REQUIRE((planes_denorm_cl || affine) && origins && dirs && depths_coarse && rgb && depth && wsum, "nfe_render_fwd: null pointer");
@@ -115,16 +114,6 @@ NFE_EXPORT int nfe_render_fwd(const nfe_render_cfg* cfg, const nfe_mlp* net_a, c
     f.scale = (float)(2.0 / (double)cfg->box_warp);
     f.origins = origins; f.dirs = dirs; f.depths = depths_coarse; f.s_per_ray = sc;
     f.m = n_rays * sc; f.total = rays * sc;
-    {   // locality ordering when the rays of an item form a square image whose side is a multiple of 4 (RaySampler's layout)
-        int64_t side = 1;
-        while (side * side < n_rays) ++side;
-        const bool square = side * side == n_rays && side % 4 == 0 && side < (1 << 15) && rays < (1ll << 32);
-        // measured on B200 (C2): L2->L1 traffic -40%, but the kernel is issue-bound and the index math costs more than
-        // the traffic saves (0.66 vs 0.62 ms), so the ordering is opt-in until the gather is memory-bound again
-        static const bool enabled = getenv("NFE_QUAD_ORDER") != nullptr;
-        f.quad_stride = (square && enabled) ? (int)side : 0;
-        f.rays_per_item = n_rays;
-    }
     f.sigma = w.sigma_c; f.rec = w.rec_c;
     f.density_noise = cfg->density_noise; f.seed = cfg->seed; f.offset = cfg->offset + 1;
     {
