@@ -36,9 +36,8 @@ const char* nfe_last_error(void);
 uint64_t nfe_launch_count(void);
 /* Measurement hook: when enabled, nfe_render_fwd / nfe_run_model_fwd bracket each stage with CUDA
  * events on the launching stream.  nfe_timing_read waits for the recorded events and returns the
- * summed milliseconds and launch counts per stage: 0 field(coarse) 1 march(coarse weights; only
- * recorded with $NFE_SPLIT_COARSE=1 — by default stage 2 forms those weights itself)
- * 2 coarse weights + resample 3 field(fine) 4 merge+composite 5 run_model. */
+ * summed milliseconds and launch counts per stage: 0 field(coarse) 1 coarse weights + resample
+ * 2 field(fine) 3 merge+composite 4 run_model. */
 int nfe_timing_enable(int on);
 int nfe_timing_read(double* ms_by_stage, int64_t* count_by_stage, int n_stages, int reset);
 

@@ -127,7 +127,7 @@ def launch_count():
     return int(load().nfe_launch_count())
 
 
-STAGES = ("field_coarse", "march_coarse", "resample", "field_fine", "march_final", "run_model")
+STAGES = ("field_coarse", "resample", "field_fine", "march_final", "run_model")
 
 
 def timing_enable(on=True):

@@ -41,10 +41,8 @@ struct MarchBwdArgs {
 
 constexpr int BWD_ARRAYS = 9;  // depth sigma w order raw alpha T dot gsm
 
-#ifndef NFE_MARCH_BWD_MIN_BLOCKS
-#define NFE_MARCH_BWD_MIN_BLOCKS 4      // 64 registers, 4 blocks per SM: 1.43 -> ~1.0 ms at c4
-#endif
-__global__ void __launch_bounds__(256, NFE_MARCH_BWD_MIN_BLOCKS) march_bwd_kernel(MarchBwdArgs a)
+constexpr int MARCH_BWD_MIN_BLOCKS = 4;   // 64 registers, 4 blocks per SM: 1.43 -> ~1.0 ms at c4
+__global__ void __launch_bounds__(256, MARCH_BWD_MIN_BLOCKS) march_bwd_kernel(MarchBwdArgs a)
 {
     extern __shared__ __align__(16) float smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;

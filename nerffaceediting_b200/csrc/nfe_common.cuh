@@ -15,8 +15,8 @@ void set_error(const char* fmt, ...);
 void count_launch();
 
 // Optional per-stage timing (nfe_timing_enable): CUDA events recorded on the launching stream.
-enum Stage { STAGE_FIELD_COARSE = 0, STAGE_MARCH_COARSE = 1, STAGE_RESAMPLE = 2, STAGE_FIELD_FINE = 3, STAGE_MARCH_FINAL = 4,
-             STAGE_RUN_MODEL = 5, STAGE_COUNT = 6 };
+enum Stage { STAGE_FIELD_COARSE = 0, STAGE_RESAMPLE = 1, STAGE_FIELD_FINE = 2, STAGE_MARCH_FINAL = 3, STAGE_RUN_MODEL = 4,
+             STAGE_COUNT = 5 };
 int stage_begin(int stage, cudaStream_t stream);   // returns a token (< 0 when timing is off)
 void stage_end(int token, cudaStream_t stream);
 struct StageScope {

@@ -3,7 +3,6 @@
 // and inverse-CDF importance resampling (sample_importance/sample_pdf, renderer.py:194-253).
 // Everything a ray needs between samples stays in the warp's shared-memory slice; cross-lane
 // work is shuffle scans.
-#include <cstdlib>
 #include "nfe_march.cuh"
 
 namespace nfe {
@@ -73,20 +72,12 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 // march_kernel: optional merge-sort of [set1 | set2] by depth, then mid-point compositing.
 //   shared slice per warp: depth[S] sigma[S] weight[S] order[S]
 // ------------------------------------------------------------------------------------------
-#ifndef NFE_MARCH_RING_DEFAULT
-#define NFE_MARCH_RING_DEFAULT 1    // merge+composite on B200: c2 0.142 -> 0.128 ms, c3 1.89 -> 1.72 ms, c5 28.7 -> 25.9 ms (4 / 12 / 16 groups: 0.135 / 0.130 / 0.143); $NFE_MARCH_RING=0 restores the register-staged loads
-#endif
-#if NFE_MARCH_FULL_WARP && !defined(NFE_MARCH_RING_GROUPS)
-#define NFE_MARCH_RING_GROUPS 3            // full-warp variant: 3 groups of 8 rows = 4.5 KB per warp
-#endif
-#ifndef NFE_MARCH_RING_GROUPS
-#define NFE_MARCH_RING_GROUPS 4            // groups (of 2*NFE_MARCH_GROUP_PAIRS rows) in a warp's record ring: 16 rows = 3 KB per warp (6 groups: no better)
-#endif
+// The packed records go through a per-warp cp.async ring (merge+composite on B200 against register-staged loads: c2 0.142 -> 0.128 ms,
+// c3 1.89 -> 1.72 ms, c5 28.7 -> 25.9 ms; 4 / 12 / 16 groups: 0.135 / 0.130 / 0.143).
+constexpr int MARCH_RING_GROUPS = 4;    // groups (of 2*MARCH_GROUP_PAIRS rows) in a warp's record ring: 16 rows = 3 KB per warp (6 groups: no better)
+constexpr int MARCH_MIN_BLOCKS = 4;     // 64 registers: 4 blocks per SM keep more record rows in flight (merge+composite at c2: 0.157 -> 0.142 ms; 5 is slower)
 template <bool SORT>
-#ifndef NFE_MARCH_MIN_BLOCKS
-#define NFE_MARCH_MIN_BLOCKS 4      // 64 registers: 4 blocks per SM keep more record rows in flight (merge+composite at c2: 0.157 -> 0.142 ms; 5 is slower)
-#endif
-__global__ void __launch_bounds__(256, NFE_MARCH_MIN_BLOCKS) march_kernel(MarchArgs a)
+__global__ void __launch_bounds__(256, MARCH_MIN_BLOCKS) march_kernel(MarchArgs a)
 {
     extern __shared__ __align__(16) float smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -102,45 +93,31 @@ __global__ void __launch_bounds__(256, NFE_MARCH_MIN_BLOCKS) march_kernel(MarchA
     for (int64_t ray_it = (int64_t)blockIdx.x * warps_per_block + warp; ray_it < a.n_rays; ray_it += (int64_t)gridDim.x * warps_per_block) {
         // Descending ray order: the records the field kernel wrote LAST are still in the 126 MB L2 when this kernel starts
         // (merge + composite at c2: 0.160 -> 0.135 ms).  Fetching a ray's records with cp.async.bulk into shared memory
-        // instead of register-staged loads was tried and is slower (0.27 ms: one 8-warp block per SM, each ray's load,
-        // weights and sums in series), so the loads below stay as they are.
+        // was tried and is slower (0.27 ms: one 8-warp block per SM, each ray's load, weights and sums in series); the
+        // per-warp cp.async ring below overlaps the record loads with the merge and the scans instead.
         const int64_t ray = a.n_rays - 1 - ray_it;
-        // ---- record ring (packed path, a.ring groups): the rows of a ray are summed in MEMORY order (sum_k omega_k c_order[k] ==
+        // ---- record ring (packed path, MARCH_RING_GROUPS groups): the rows of a ray are summed in MEMORY order (sum_k omega_k c_order[k] ==
         //      sum_e omega'_e c_e with omega' scattered by entry), so their addresses are known before the merge: the first
-        //      a.ring groups (two rows each) are requested here with cp.async and land while the merge and the scans run
+        //      MARCH_RING_GROUPS groups are requested here with cp.async and land while the merge and the scans run
         const int rg_half = lane >> 4, rg_q = lane & 15;
         const bool rg_on = rg_q < 12;
         const float4* rg_r1 = nullptr;
         const float4* rg_r2 = nullptr;
         uint32_t rg_slot0 = 0;
-        if (a.ring) {
+        if (a.rec1) {
             rg_r1 = reinterpret_cast<const float4*>(a.rec1 + ray * a.s1 * 48) + rg_q;
             rg_r2 = a.s2 ? reinterpret_cast<const float4*>(a.rec2 + (ray * a.s2 - a.s1) * 48) + rg_q : rg_r1;
             char* ring_base = reinterpret_cast<char*>(smem) + (((size_t)warps_per_block * MARCH_SMEM_FLOATS_PER_SAMPLE * S * 4 + 15) & ~(size_t)15)
-                              + (size_t)warp * a.ring * MARCH_RING_GROUP_BYTES;
-#if NFE_MARCH_FULL_WARP
-            // chunk c = lane + 32 j (j = 0..2) of a group's 96 chunks: row c / 12 of the group, 16-byte piece c % 12 of that row
-            rg_r1 -= rg_q; rg_r2 -= rg_q;
-            rg_slot0 = (uint32_t)__cvta_generic_to_shared(ring_base) + (uint32_t)(lane * 16);
-            for (int g = 0; g < a.ring; ++g) {
-#pragma unroll
-                for (int j = 0; j < 3; ++j) {
-                    const int c = lane + 32 * j, e = 8 * g + c / 12;
-                    if (e < S) cp_async16(rg_slot0 + g * MARCH_RING_GROUP_BYTES + j * 512, (e < a.s1 ? rg_r1 : rg_r2) + e * 12 + c % 12);
-                }
-                cp_async_commit();
-            }
-#else
+                              + (size_t)warp * MARCH_RING_GROUPS * MARCH_RING_GROUP_BYTES;
             rg_slot0 = (uint32_t)__cvta_generic_to_shared(ring_base) + (uint32_t)(rg_half * 192 + rg_q * 16);
-            for (int g = 0; g < a.ring; ++g) {
+            for (int g = 0; g < MARCH_RING_GROUPS; ++g) {
 #pragma unroll
-                for (int j = 0; j < NFE_MARCH_GROUP_PAIRS; ++j) {
-                    const int e = 2 * (NFE_MARCH_GROUP_PAIRS * g + j) + rg_half;
+                for (int j = 0; j < MARCH_GROUP_PAIRS; ++j) {
+                    const int e = 2 * (MARCH_GROUP_PAIRS * g + j) + rg_half;
                     if (rg_on && e < S) cp_async16(rg_slot0 + g * MARCH_RING_GROUP_BYTES + j * 384, (e < a.s1 ? rg_r1 : rg_r2) + e * 12);
                 }
                 cp_async_commit();
             }
-#endif
         }
         // ---- load (and merge) depths / densities
         if (SORT) {
@@ -208,117 +185,38 @@ __global__ void __launch_bounds__(256, NFE_MARCH_MIN_BLOCKS) march_kernel(MarchA
         // ---- channel sums
         if (a.rec1) {
             // Packed records (48 floats = 12 float4 per sample): a half-warp reads one whole 192-byte row per load,
-            // lanes 0-11 take row k, lanes 16-27 row k+1; the two halves are added at the end.
+            // lanes 0-11 take the even rows, lanes 16-27 the odd ones; the two halves are added at the end.
             for (int k = lane; k < S; k += 32) s_sigma[k] = 0.5f * ((k > 0 ? s_w[k - 1] : 0.0f) + (k < n_int ? s_w[k] : 0.0f));
             __syncwarp();
             const int half = lane >> 4, q = lane & 15;
             const bool on = q < 12;
-            const float4* r1 = reinterpret_cast<const float4*>(a.rec1 + ray * a.s1 * 48) + (on ? q : 0);
-            const float4* r2 = a.s2 ? reinterpret_cast<const float4*>(a.rec2 + (ray * a.s2 - a.s1) * 48) + (on ? q : 0) : r1;
             float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-            constexpr int UN = 4;                              // 8 rows in flight per warp
-            int k0 = 0;
-            if (a.ring) {
-                // omega by entry (s_raw is free after the merge), then walk the ring: group g holds 2*NFE_MARCH_GROUP_PAIRS consecutive rows in memory order;
-                // every lane reads back exactly the 16 bytes it requested itself, so cp.async.wait_group is all the ordering needed
-                for (int k = lane; k < S; k += 32) s_raw[s_order[k]] = s_sigma[k];
-                __syncwarp();
-#if NFE_MARCH_FULL_WARP
-                float4 part[3];
+            // omega by entry (s_raw is free after the merge), then walk the ring: group g holds 2*MARCH_GROUP_PAIRS consecutive rows in memory order;
+            // every lane reads back exactly the 16 bytes it requested itself, so cp.async.wait_group is all the ordering needed
+            for (int k = lane; k < S; k += 32) s_raw[s_order[k]] = s_sigma[k];
+            __syncwarp();
+            const int n_groups = (S + 2 * MARCH_GROUP_PAIRS - 1) / (2 * MARCH_GROUP_PAIRS);
+            int slot = 0;
+            for (int g = 0; g < n_groups; ++g) {
+                cp_async_wait<MARCH_RING_GROUPS - 1>();       // MARCH_RING_GROUPS groups were committed after group g-1: g has landed
 #pragma unroll
-                for (int j = 0; j < 3; ++j) part[j] = make_float4(0.f, 0.f, 0.f, 0.f);
-                const int n_groups8 = (S + 7) >> 3;
-                int slot8 = 0;
-                for (int g = 0; g < n_groups8; ++g) {
-                    cp_async_wait<NFE_MARCH_RING_GROUPS - 1>();
-#pragma unroll
-                    for (int j = 0; j < 3; ++j) {
-                        const int c = lane + 32 * j, e = 8 * g + c / 12;
-                        if (e < S) {
-                            float4 v;
-                            asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w)
-                                         : "r"(rg_slot0 + slot8 * MARCH_RING_GROUP_BYTES + j * 512) : "memory");
-                            const float om = s_raw[e];
-                            part[j].x = fmaf(om, v.x, part[j].x); part[j].y = fmaf(om, v.y, part[j].y);
-                            part[j].z = fmaf(om, v.z, part[j].z); part[j].w = fmaf(om, v.w, part[j].w);
-                        }
-                    }
-#pragma unroll
-                    for (int j = 0; j < 3; ++j) {   // refill the slot just consumed
-                        const int c = lane + 32 * j, e2 = 8 * (g + a.ring) + c / 12;
-                        if (e2 < S) cp_async16(rg_slot0 + slot8 * MARCH_RING_GROUP_BYTES + j * 512, (e2 < a.s1 ? rg_r1 : rg_r2) + e2 * 12 + c % 12);
-                    }
-                    cp_async_commit();
-                    slot8 = slot8 + 1 == a.ring ? 0 : slot8 + 1;
-                }
-                // (lane, j) holds the partial sums of piece (lane + 32 j) % 12: fold the 96 partials through the (now idle) first ring slot;
-                // lanes 0-11 end up with the totals of piece q = lane, which is what the output code below expects of the lower half-warp
-                cp_async_wait<0>();
-#pragma unroll
-                for (int j = 0; j < 3; ++j)
-                    asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(rg_slot0 + j * 512), "f"(part[j].x), "f"(part[j].y), "f"(part[j].z), "f"(part[j].w) : "memory");
-                __syncwarp();
-                if (lane < 12) {
-#pragma unroll
-                    for (int r = 0; r < 8; ++r) {
+                for (int j = 0; j < MARCH_GROUP_PAIRS; ++j) {
+                    const int e = 2 * (MARCH_GROUP_PAIRS * g + j) + rg_half;
+                    if (rg_on && e < S) {
                         float4 v;
                         asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w)
-                                     : "r"(rg_slot0 + r * 192) : "memory");
-                        acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
+                                     : "r"(rg_slot0 + slot * MARCH_RING_GROUP_BYTES + j * 384) : "memory");
+                        const float om = s_raw[e];
+                        acc.x = fmaf(om, v.x, acc.x); acc.y = fmaf(om, v.y, acc.y); acc.z = fmaf(om, v.z, acc.z); acc.w = fmaf(om, v.w, acc.w);
                     }
                 }
-                __syncwarp();
-#else
-                const int n_groups = (S + 2 * NFE_MARCH_GROUP_PAIRS - 1) / (2 * NFE_MARCH_GROUP_PAIRS);
-                int slot = 0;
-                for (int g = 0; g < n_groups; ++g) {
-                    cp_async_wait<NFE_MARCH_RING_GROUPS - 1>();       // a.ring == NFE_MARCH_RING_GROUPS groups were committed after group g-1: g has landed
 #pragma unroll
-                    for (int j = 0; j < NFE_MARCH_GROUP_PAIRS; ++j) {
-                        const int e = 2 * (NFE_MARCH_GROUP_PAIRS * g + j) + rg_half;
-                        if (rg_on && e < S) {
-                            float4 v;
-                            asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w)
-                                         : "r"(rg_slot0 + slot * MARCH_RING_GROUP_BYTES + j * 384) : "memory");
-                            const float om = s_raw[e];
-                            acc.x = fmaf(om, v.x, acc.x); acc.y = fmaf(om, v.y, acc.y); acc.z = fmaf(om, v.z, acc.z); acc.w = fmaf(om, v.w, acc.w);
-                        }
-                    }
-#pragma unroll
-                    for (int j = 0; j < NFE_MARCH_GROUP_PAIRS; ++j) {   // refill the slot just consumed
-                        const int e2 = 2 * (NFE_MARCH_GROUP_PAIRS * (g + a.ring) + j) + rg_half;
-                        if (rg_on && e2 < S) cp_async16(rg_slot0 + slot * MARCH_RING_GROUP_BYTES + j * 384, (e2 < a.s1 ? rg_r1 : rg_r2) + e2 * 12);
-                    }
-                    cp_async_commit();
-                    slot = slot + 1 == a.ring ? 0 : slot + 1;
+                for (int j = 0; j < MARCH_GROUP_PAIRS; ++j) {   // refill the slot just consumed
+                    const int e2 = 2 * (MARCH_GROUP_PAIRS * (g + MARCH_RING_GROUPS) + j) + rg_half;
+                    if (rg_on && e2 < S) cp_async16(rg_slot0 + slot * MARCH_RING_GROUP_BYTES + j * 384, (e2 < a.s1 ? rg_r1 : rg_r2) + e2 * 12);
                 }
-#endif
-                k0 = S;                                        // the register-staged loops below are skipped
-            }
-            for (; k0 + 2 * UN <= S; k0 += 2 * UN) {
-                float4 v[UN];
-                float om[UN];
-#pragma unroll
-                for (int u = 0; u < UN; ++u) {
-                    const int k = k0 + 2 * u + half;
-                    const int e = s_order[k];
-                    v[u] = __ldg((e < a.s1 ? r1 : r2) + e * 12);
-                    om[u] = s_sigma[k];
-                }
-#pragma unroll
-                for (int u = 0; u < UN; ++u) {
-                    acc.x = fmaf(om[u], v[u].x, acc.x); acc.y = fmaf(om[u], v[u].y, acc.y);
-                    acc.z = fmaf(om[u], v[u].z, acc.z); acc.w = fmaf(om[u], v[u].w, acc.w);
-                }
-            }
-            for (; k0 < S; k0 += 2) {
-                const int k = k0 + half;
-                if (k < S) {
-                    const int e = s_order[k];
-                    const float4 v = __ldg((e < a.s1 ? r1 : r2) + e * 12);
-                    const float om = s_sigma[k];
-                    acc.x = fmaf(om, v.x, acc.x); acc.y = fmaf(om, v.y, acc.y); acc.z = fmaf(om, v.z, acc.z); acc.w = fmaf(om, v.w, acc.w);
-                }
+                cp_async_commit();
+                slot = slot + 1 == MARCH_RING_GROUPS ? 0 : slot + 1;
             }
             acc.x += __shfl_xor_sync(0xffffffffu, acc.x, 16); acc.y += __shfl_xor_sync(0xffffffffu, acc.y, 16);
             acc.z += __shfl_xor_sync(0xffffffffu, acc.z, 16); acc.w += __shfl_xor_sync(0xffffffffu, acc.w, 16);
@@ -478,14 +376,12 @@ __global__ void __launch_bounds__(256) unify_kernel(MarchArgs a, float* __restri
 // fp32, the CDF a double running sum rounded per entry.  No fused multiply-adds.
 //   shared slice per warp: z[S] a[S] bins[S] cdf[S]
 // ------------------------------------------------------------------------------------------
+constexpr int RESAMPLE_MIN_BLOCKS = 4;  // with the coarse weights fused in (c2): 3 blocks 0.060 ms, 4 blocks 0.049 ms (16 bytes of spill), 6 blocks 0.053 ms
 // SMOOTH = true : sample_importance — inputs are z_vals [S] and raw coarse weights [S-1];
 //                 ns = S-3 pdf entries, bins = the S-1 mid-depths.
 // SMOOTH = false: sample_pdf stand-alone — inputs are bins [S] and weights [ns] as given.
 template <bool SMOOTH>
-#ifndef NFE_RESAMPLE_MIN_BLOCKS
-#define NFE_RESAMPLE_MIN_BLOCKS 4   // with the coarse weights fused in (c2): 3 blocks 0.060 ms, 4 blocks 0.049 ms (16 bytes of spill), 6 blocks 0.053 ms
-#endif
-__global__ void __launch_bounds__(256, NFE_RESAMPLE_MIN_BLOCKS) resample_kernel(ResampleArgs a)
+__global__ void __launch_bounds__(256, RESAMPLE_MIN_BLOCKS) resample_kernel(ResampleArgs a)
 {
     extern __shared__ __align__(16) float smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -610,21 +506,17 @@ int launch_march(const MarchArgs& a, bool sort, cudaStream_t stream)
     if (a.n_rays <= 0) return 0;
     const int warps = warps_for(S, MARCH_SMEM_FLOATS_PER_SAMPLE);
     size_t smem = (size_t)warps * MARCH_SMEM_FLOATS_PER_SAMPLE * 4 * S;
-    MarchArgs args = a;
-    // packed records: cp.async ring of NFE_MARCH_RING_GROUPS groups per warp behind the scan arrays ($NFE_MARCH_RING=0 keeps the
-    // register-staged loads)
-    static const bool ring_on = [] { const char* e = getenv("NFE_MARCH_RING"); return e ? atoi(e) != 0 : NFE_MARCH_RING_DEFAULT != 0; }();
-    args.ring = (a.rec1 && ring_on) ? NFE_MARCH_RING_GROUPS : 0;
-    if (args.ring) smem = ((smem + 15) & ~(size_t)15) + (size_t)warps * args.ring * MARCH_RING_GROUP_BYTES;
+    // packed records: cp.async ring of MARCH_RING_GROUPS groups per warp behind the scan arrays
+    if (a.rec1) smem = ((smem + 15) & ~(size_t)15) + (size_t)warps * MARCH_RING_GROUPS * MARCH_RING_GROUP_BYTES;
     const int64_t blocks = (a.n_rays + warps - 1) / warps;
     const int64_t cap = (int64_t)sm_count() * 8;
     const unsigned grid = (unsigned)(blocks < cap ? blocks : cap);
     if (sort) {
         if (smem > SMEM_OPT_IN) cudaFuncSetAttribute(march_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        march_kernel<true><<<grid, warps * 32, smem, stream>>>(args);
+        march_kernel<true><<<grid, warps * 32, smem, stream>>>(a);
     } else {
         if (smem > SMEM_OPT_IN) cudaFuncSetAttribute(march_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        march_kernel<false><<<grid, warps * 32, smem, stream>>>(args);
+        march_kernel<false><<<grid, warps * 32, smem, stream>>>(a);
     }
     return check_launch("march_kernel");
 }

@@ -5,17 +5,8 @@
 namespace nfe {
 
 constexpr int MARCH_SMEM_FLOATS_PER_SAMPLE = 5;  // depth, sigma, weight, order, unsorted sigma
-#ifndef NFE_MARCH_GROUP_PAIRS
-#define NFE_MARCH_GROUP_PAIRS 2   // row pairs per ring group (one cp.async per lane and pair); 2 halves the wait/commit/loop overhead per row: same box, 0.138 -> 0.125 ms
-#endif
-#ifndef NFE_MARCH_FULL_WARP
-#define NFE_MARCH_FULL_WARP 0     // untested next-round variant: groups of 8 rows = 96 16-byte chunks, three per lane, all 32 lanes busy
-#endif
-#if NFE_MARCH_FULL_WARP
-constexpr int MARCH_RING_GROUP_BYTES = 8 * 192;
-#else
-constexpr int MARCH_RING_GROUP_BYTES = NFE_MARCH_GROUP_PAIRS * 2 * 192;  // one ring group = pairs of 192-byte record rows (one row per half-warp)
-#endif
+constexpr int MARCH_GROUP_PAIRS = 2;  // row pairs per ring group (one cp.async per lane and pair); 2 halves the wait/commit/loop overhead per row: same box, 0.138 -> 0.125 ms
+constexpr int MARCH_RING_GROUP_BYTES = MARCH_GROUP_PAIRS * 2 * 192;  // one ring group = pairs of 192-byte record rows (one row per half-warp)
 constexpr int MAX_S = 768;  // merged samples per ray (reference configs go up to 192+192, SURVEY.md §8a)
 
 struct MarchArgs {
@@ -30,7 +21,6 @@ struct MarchArgs {
     int64_t image_rays; // packed path only: > 0 writes rgb / seg as images [item, channel, image_rays] instead of [ray, channel]
     int inputs_sorted; // both sample sets ascending in depth: merge by binary search instead of a full rank sort
     int white_back;
-    int ring;          // packed path only (set by launch_march): groups of the per-warp cp.async record ring, 0 = register-staged loads
     float* rgb;        // [n_rays,cc]
     float* seg;        // [n_rays,cs]
     float* depth;      // [n_rays], UNCLAMPED (finish_depth applies the global clamp)

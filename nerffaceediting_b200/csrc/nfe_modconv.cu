@@ -46,17 +46,11 @@
 #include "nfe_tc.cuh"
 
 namespace nfe {
-#ifndef NFE_MC_SEG_Q
-#define NFE_MC_SEG_Q 4
-#endif
 namespace mc {
 
-#ifdef NFE_MC_EXP_ALIGNED      // timing experiment only (wrong results): window rows at a 128-byte pitch, no column shifts
-constexpr int HALO_W = 8;
-#else
 constexpr int HALO_W = 10;
-#endif
 constexpr int TILE_W = 8, MAX_TAPS = 9, THREADS = 256, MAX_SA = 4, MAX_SB = 6;
+constexpr int SEG_Q16 = 4;                                // epilogue segment: 4 groups of 16 fp16 columns = 128 bytes of a staged row
 
 constexpr int TABLE_BYTES = 256 + 1024 + 1024 + 128;      // mbarriers + TMEM slot | bias of the N tile | output scale of the N tile | tap tables
 constexpr int SMEM_BUDGET = 227 * 1024 - TABLE_BYTES;
@@ -124,11 +118,6 @@ __device__ __forceinline__ void bulk_copy(void* dst, const void* src, uint32_t b
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                  :: "r"(tc::smem_u32(dst)), "l"(src), "r"(bytes), "r"(tc::smem_u32(bar)) : "memory");
 }
-// bulk copy shared -> global (TMA unit), tracked by the issuing thread's bulk groups
-__device__ __forceinline__ void bulk_store(void* gdst, const void* ssrc, uint32_t bytes)
-{
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" :: "l"(gdst), "r"(tc::smem_u32(ssrc)), "r"(bytes) : "memory");
-}
 __device__ __forceinline__ void sts128(uint32_t addr, uint32_t x, uint32_t y, uint32_t z, uint32_t w)
 {
     asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" :: "r"(addr), "r"(x), "r"(y), "r"(z), "r"(w) : "memory");
@@ -145,9 +134,6 @@ __device__ __forceinline__ float fmax3(float a, float b, float c)
     asm("max.f32 %0, %1, %2, %3;" : "=f"(r) : "f"(a), "f"(b), "f"(c));      // FMNMX3 (sm_100)
     return r;
 }
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
 // one lane of the (converged) warp; the callers keep their control flow warp-uniform so that descriptors and barrier addresses
 // live in uniform registers: a divergent `if (lane == 0)` loop makes the compiler wrap every tcgen05.mma in an ELECT / R2UR
@@ -252,11 +238,7 @@ __global__ void __launch_bounds__(PS ? PS_THREADS : THREADS, (!PS && MA == 1 && 
     }
     if (warp == MMA_WARP) tc::tmem_alloc(tmem_slot, tmem_cols);
     if (threadIdx.x < MAX_TAPS) {
-#ifdef NFE_MC_EXP_ALIGNED
-        s_tap16[threadIdx.x] = (uint32_t)((1 + tp.dy[tp.blk_tap[threadIdx.x]]) * HALO_W);
-#else
         s_tap16[threadIdx.x] = (uint32_t)((1 + tp.dy[tp.blk_tap[threadIdx.x]]) * HALO_W + 1 + tp.dx[tp.blk_tap[threadIdx.x]]);
-#endif
         s_tmask[threadIdx.x] = tp.acc_mask[tp.blk_tap[threadIdx.x]] | (tp.blk_width[threadIdx.x] == 2 ? 0x100u : 0u);      // per BLOCK; bit 8: two taps wide
     }
     if (threadIdx.x < MAX_ACC) s_row16[threadIdx.x] = (uint32_t)(tp.row_off[threadIdx.x] * (HALO_W * 16)) >> 4;
@@ -373,11 +355,7 @@ __global__ void __launch_bounds__(PS ? PS_THREADS : THREADS, (!PS && MA == 1 && 
         // the tensor core's 64-128 cycles per instruction.  Every lane runs the loop; one elected lane issues.
         {
             const bool leader = elect_one();
-#ifdef NFE_MC_EXP_FMT0
-            const uint32_t idesc = make_idesc(128, a.n_tile, 0);
-#else
             const uint32_t idesc = make_idesc(128, a.n_tile, PARTS == 1 ? 0 : 1);
-#endif
             const uint32_t b_lbo = a.n_tile * 16, b_part16 = (a.n_tile * a.kc * 2) >> 4, a_part16 = A_PART >> 4;
             const uint64_t da0 = tc::make_desc(0, A_LBO, A_SBO), db0 = tc::make_desc(0, b_lbo, 128);
             const uint32_t a_k16 = (2 * A_LBO) >> 4, b_k16 = (2 * b_lbo) >> 4;
@@ -390,11 +368,7 @@ __global__ void __launch_bounds__(PS ? PS_THREADS : THREADS, (!PS && MA == 1 && 
             // cycles per MMA measured there against the 143 of the (already 7 k instruction) fp16 build.
             int sb = 0;
             uint32_t sb_par = 0;
-#ifdef NFE_MC_EXP_TERMS1
-            constexpr int TERMS = 1;
-#else
             constexpr int TERMS = PARTS == 2 ? 3 : 1;
-#endif
 #pragma unroll 1
             for (int k = 0, g = 0; k < n_win; ++k) {
             uint32_t started = 0;                    // accumulators that hold a partial sum already
@@ -518,22 +492,19 @@ __global__ void __launch_bounds__(PS ? PS_THREADS : THREADS, (!PS && MA == 1 && 
         // 32 finished rows out with coalesced 16-byte stores (16 or 32 lanes per row): warp-local, no block-wide synchronisation.
         // (Round 2 first handed each row to the TMA unit as a bulk store; a per-thread cp.async.bulk compiles to a 32-trip waterfall
         // around a uniform-datapath UBLKCP.  Both variants take the same time — the SM's store path is the limit —; the copy-out needs
-        // no async-proxy fences and no wait before a row is reused.  -DNFE_MC_BULK_EPILOGUE keeps the bulk variant for the A/B record,
+        // no async-proxy fences and no wait before a row is reused.  The bulk variant was measured and removed:
         // profiles/modconv_tuning_r02.txt #13.)
-        // Segments are short (NFE_MC_SEG_Q groups = 64 columns): the stage then needs 144-272 bytes per row instead of 528 and fits
+        // Segments are short (SEG_Q16 fp16 groups = 64 columns): the stage then needs 144-272 bytes per row instead of 528 and fits
         // beside every CTA shape.  (Measured: an SM's stores leave at ~28 bytes per clock — 16 KB per warp in ~4.8 k cycles with 8 warps
         // storing — and segment length does not change the epilogue's length: the stores hold the warp, a segment does not drain
         // behind the next one's arithmetic.  profiles/modconv_tuning_r02.txt #13.)
-        constexpr int SEG_Q = NFE_MC_SEG_Q * 2 / (int)sizeof(T);                     // 16-column groups per segment: 128 bytes of a row
+        constexpr int SEG_Q = SEG_Q16 * 2 / (int)sizeof(T);                          // 16-column groups per segment: 128 bytes of a row
         const int PITCH = min(a.n_tile, SEG_Q * 16) * (int)sizeof(T) + 16;           // row pitch in the stage
         const bool staged = vec_ok && a.stage_ok && (nt + 1) * a.n_tile <= a.out_ch;
         // (the persistent CTA's rings are busy with the next window: its stage is a region of its own behind the tables)
         const uint32_t stage0 = tc::smem_u32(smem) + (PS ? (uint32_t)(SA * A_STAGE + a.sb * a.b_slot + TABLE_BYTES) : 0u);
         const uint32_t warp_rows = stage0 + (uint32_t)((grp * 128 + (ew & 3) * 32) * PITCH);    // this warp's 32 staged rows
         const uint32_t my_row = warp_rows + (uint32_t)(lane * PITCH);
-#ifdef NFE_MC_BULK_EPILOGUE
-        bool pending = false;                                                        // a bulk store of my_row may still be reading it
-#endif
         // The epilogue is bound by its instruction count (8 warps x n_tile / 16 groups of 16 columns; ncu: 60 % of the kernel's executed
         // instructions at 256 x 256 channels).  Per value: (v + noise) + bias as packed f32x2 adds, the slope pair as max(t g+, t g-) —
         // equal to t * (t > 0 ? g+ : g-) for gain > 0 and 0 <= slope <= 1 — folded with the lower clamp into one three-input max,
@@ -557,14 +528,6 @@ __global__ void __launch_bounds__(PS ? PS_THREADS : THREADS, (!PS && MA == 1 && 
             // the segment just completed in the warp's staged rows goes out: (qs + 1) * 16 columns = `pieces` 16-byte pieces per row;
             // lane i takes piece i % pieces of row i / pieces, then 32 further on, ...: a store instruction covers whole rows
             auto copy_out = [&](const int q, const int qs) {
-#ifdef NFE_MC_BULK_EPILOGUE
-                if (valid) {
-                    tc::fence_async_smem();             // this thread's row, written through the generic proxy, is read by the async proxy
-                    bulk_store(dst + (q - qs) * 16, reinterpret_cast<const void*>(__cvta_shared_to_generic(my_row)), (uint32_t)((qs + 1) * 16 * (int)sizeof(T)));
-                    bulk_commit();
-                    pending = true;
-                }
-#else
                 // (`slots` = pieces rounded up to a power of two: lanes whose slot is past the row's pieces sit a trip out — only a tile
                 //  of 48, 112, ... channels has such a segment)
                 const int pieces = (qs + 1) * (int)sizeof(T), shift = 32 - __clz(pieces - 1), slots = 1 << shift;       // pieces 2 .. 16
@@ -589,7 +552,6 @@ __global__ void __launch_bounds__(PS ? PS_THREADS : THREADS, (!PS && MA == 1 && 
                         if (d[k]) *reinterpret_cast<uint4*>(d[k] + seg_off + pcs[k] * 16) = u[k];
                 }
                 __syncwarp();                          // the rows are rewritten by the next segment
-#endif
             };
             auto stage = [&](const int qs, const float (&v)[16]) {
                 // (rows outside the image are staged too and skipped by the copy-out: the warp stays converged)
@@ -610,9 +572,6 @@ __global__ void __launch_bounds__(PS ? PS_THREADS : THREADS, (!PS && MA == 1 && 
                 // ---- the production path: staged rows, packed math, two register arrays
                 auto group = [&](const int q, float (&v)[16]) {
                     const int qs = q % SEG_Q;
-#ifdef NFE_MC_BULK_EPILOGUE
-                    if (qs == 0 && pending) { bulk_wait_read(); pending = false; }      // the row buffer is free once the previous store has read it
-#endif
                     if (!raw) {
 #pragma unroll
                         for (int i4 = 0; i4 < 4; ++i4) {
@@ -674,9 +633,6 @@ __global__ void __launch_bounds__(PS ? PS_THREADS : THREADS, (!PS && MA == 1 && 
                 }
             }
         }
-#ifdef NFE_MC_BULK_EPILOGUE
-        if (staged) bulk_wait_read();                       // shared memory must outlive the reads; the writes complete with the kernel
-#endif
         tc::fence_before_sync();
         if constexpr (PS) {                                // tensor memory is free for the next window's MMAs
             __syncwarp();
@@ -915,12 +871,10 @@ __global__ void __launch_bounds__(256) upfir_finish_kernel(const FinishArgs a)
 // above re-reads every input pixel 16 times through L1 / L2: measured 3x the time the bytes need) and then every thread computes
 // 16 bytes of channels per output pixel from 16-byte shared-memory reads.
 constexpr int FT = 16, FT_IN = FT + 3;
+constexpr int FIN_MIN_BLOCKS = 4;
 
-#ifndef NFE_FIN_MIN_BLOCKS
-#define NFE_FIN_MIN_BLOCKS 4
-#endif
 template <class T>
-__global__ void __launch_bounds__(256, NFE_FIN_MIN_BLOCKS) upfir_finish_tiled_kernel(const FinishArgs a, int tiles_x, int tiles_y, int slices)
+__global__ void __launch_bounds__(256, FIN_MIN_BLOCKS) upfir_finish_tiled_kernel(const FinishArgs a, int tiles_x, int tiles_y, int slices)
 {
     constexpr int V = 16 / (int)sizeof(T);                   // channels per 16 bytes
     __shared__ __align__(16) unsigned char tile[FT_IN * FT_IN * 128];
@@ -1211,10 +1165,9 @@ static int make_plan(const nfe_modconv_args& q, Plan& pl)
     //  * a LARGE fp16 layer of N <= 128 does better still as persistent window pairs (below): two 128-column accumulators are half of
     //    tensor memory, so a persistent CTA has TWO sets and issues window k + 1 while the epilogue reads window k out — the overlap the
     //    twin CTAs give, plus shared weight stages and no per-window start-up (128->128 at 512^2: 0.77 -> 0.64 ms; with split operands
-    //    the same change measured slower, fp32 SR head 5.64 -> 5.85 ms, so fp32 keeps the twins).  $NFE_MC_PERSIST_N128=0: twins always.
-    static const bool ps_n128_on = [] { const char* e = getenv("NFE_MC_PERSIST_N128"); return e ? atoi(e) != 0 : true; }();
+    //    the same change measured slower, fp32 SR head 5.64 -> 5.85 ms, so fp32 keeps the twins).
     const bool twin0 = q.up == 1 && pl.n_tile <= 128 && !one_by_one && (pl.parts == 1 || can32);
-    const bool twin = twin0 && !(ps_n128_on && pl.parts == 1 && ctas_256 >= 3ll * sm_count());
+    const bool twin = twin0 && !(pl.parts == 1 && ctas_256 >= 3ll * sm_count());
     const bool pair = q.up == 1 && !twin && ((pl.parts == 1 && (ctas_256 >= sm_count() || one_by_one)) ||
                                              (pl.parts == 2 && can32 && !one_by_one && ctas_256 >= sm_count()));
     // (up = 2 with split operands: blocks of two taps are 64 KB at 64-channel chunks and the ring holds two; 32-channel chunks — five
@@ -1272,9 +1225,8 @@ static int make_plan(const nfe_modconv_args& q, Plan& pl)
         pl.grid_h = q.in_h + 1; pl.grid_w = q.in_w + 1;
     }
     // weight blocks: taps in order; a tap takes along a later one that reads the same shifted window, feeds the next accumulator (same
-    // window rows) and finds it in the same state (both fresh or both started) — see TapPlan.  $NFE_MC_MERGE=0 keeps one tap per block.
+    // window rows) and finds it in the same state (both fresh or both started) — see TapPlan.
     {
-        static const bool merge_on = [] { const char* e = getenv("NFE_MC_MERGE"); return e ? atoi(e) != 0 : true; }();
         auto single = [](unsigned m) { return m && !(m & (m - 1)); };
         auto bit = [](unsigned m) { int b = 0; while (!((m >> b) & 1u)) ++b; return b; };
         bool used[MAX_TAPS] = {};
@@ -1287,9 +1239,8 @@ static int make_plan(const nfe_modconv_args& q, Plan& pl)
             p.blk_tap[u] = t; p.blk_width[u] = 1; p.blk_unit[u] = unit; p.tap_blk[t] = u; p.tap_half[t] = 0;
             used[t] = true;
             // (split operands: a two-tap block is 64 KB at 64-channel chunks, the ring then holds two and the CTA cannot be persistent;
-            //  merging still measured faster — fp32 SR head 5.52 vs 5.58 ms, 32->256 up=2 0.49 vs 0.55 ms.  $NFE_MC_MERGE_SPLIT=0: do not)
-            static const bool merge_split = [] { const char* e = getenv("NFE_MC_MERGE_SPLIT"); return e ? atoi(e) != 0 : true; }();
-            if (merge_on && (pl.parts == 1 || merge_split) && q.up == 2 && 2 * pl.n_tile <= 256 && single(p.acc_mask[t])) {
+            //  merging still measured faster — fp32 SR head 5.52 vs 5.58 ms, 32->256 up=2 0.49 vs 0.55 ms)
+            if (q.up == 2 && 2 * pl.n_tile <= 256 && single(p.acc_mask[t])) {
                 const int m = bit(p.acc_mask[t]);
                 for (int t2 = t + 1; t2 < p.taps && m + 1 < p.n_acc; ++t2) {
                     if (used[t2] || p.dy[t2] != p.dy[t] || p.dx[t2] != p.dx[t] || p.acc_mask[t2] != (1u << (m + 1))) continue;
@@ -1311,14 +1262,13 @@ static int make_plan(const nfe_modconv_args& q, Plan& pl)
         pl.sb = std::min(MAX_SB, (budget - a_bytes) / pl.b_slot);
         NFE_REQUIRE(pl.sb >= 2, "nfe_modulated_conv2d: internal: weight ring does not fit");
         // epilogue stage: two warp groups x 128 rows of one 128-byte segment (+ 16 bytes of pitch)
-        pl.stage_bytes = 2 * 128 * (std::min(pl.n_tile * (pl.parts == 1 ? 2 : 4), NFE_MC_SEG_Q * 32) + 16);
+        pl.stage_bytes = 2 * 128 * (std::min(pl.n_tile * (pl.parts == 1 ? 2 : 4), SEG_Q16 * 32) + 16);
         // Persistent CTAs (conv_gemm_kernel<..., PS = true>) where one CTA fills the SM anyway (twin CTAs overlap each other already),
-        // every SM gets several windows, and the weight ring keeps three slots beside the stage region.  $NFE_MC_PERSIST=0: never.
-        static const bool persist_on = [] { const char* e = getenv("NFE_MC_PERSIST"); return e ? atoi(e) != 0 : true; }();
+        // every SM gets several windows, and the weight ring keeps three slots beside the stage region.
         const long long items = (long long)((q.up == 2 ? q.in_h + 1 : q.in_h) + 16 * pl.ma - 1) / (16 * pl.ma) *
                                 (((q.up == 2 ? q.in_w + 1 : q.in_w) + TILE_W - 1) / TILE_W) * pl.n_tiles * q.batch;
         const int sb_ps = std::min(MAX_SB, (budget - a_bytes - pl.stage_bytes) / pl.b_slot);
-        pl.persist = persist_on && !twin && items >= 3ll * sm_count() && items < (1ll << 30) && sb_ps >= 3;
+        pl.persist = !twin && items >= 3ll * sm_count() && items < (1ll << 30) && sb_ps >= 3;
         if (pl.persist) pl.sb = sb_ps;
     }
     pl.packed_item_bytes = (long long)pl.n_tiles * pl.chunks * p.taps * pl.b_stage;
@@ -1433,9 +1383,8 @@ NFE_EXPORT int nfe_modulated_conv2d(const nfe_modconv_args* q, void* workspace, 
     // Split operands (fp32) with one weight for the batch: pack W ONCE and let the GEMM carry the style (on the activations, in the halo
     // loader) and the demodulation coefficient (on the accumulator, in the epilogue) — the reference's non-fused formulation,
     // networks_stylegan2.py:69-79, equal to the fused one up to fp32 rounding order.  The per-item pack wrote batch x the weight tensor
-    // (hi + lo) per layer call: 0.47 ms of a 5.2 ms fp32 backbone pass.  $NFE_MC_SHARED_W=0 keeps per-item weights.
-    static const bool shared_on = [] { const char* e = getenv("NFE_MC_SHARED_W"); return e ? atoi(e) != 0 : true; }();
-    const bool shared = shared_on && pl.parts == 2 && q->weight_batch_stride == 0 && q->batch > 1 && (reinterpret_cast<uintptr_t>(q->styles) & 15) == 0;
+    // (hi + lo) per layer call: 0.47 ms of a 5.2 ms fp32 backbone pass.
+    const bool shared = pl.parts == 2 && q->weight_batch_stride == 0 && q->batch > 1 && (reinterpret_cast<uintptr_t>(q->styles) & 15) == 0;
     pa.shared = shared ? 1 : 0;
     NFE_REQUIRE(q->in_ch <= 8192, "nfe_modulated_conv2d: in_channels above 8192");
     mc::modconv_coef_kernel<<<q->out_ch, 128, (size_t)q->in_ch * sizeof(float), stream>>>(pa);
@@ -1451,7 +1400,7 @@ NFE_EXPORT int nfe_modulated_conv2d(const nfe_modconv_args* q, void* workspace, 
     g.n_tile = pl.n_tile; g.n_tiles = pl.n_tiles; g.chunks = pl.chunks; g.kc = pl.kc; g.sb = pl.sb; g.b_stage = pl.b_stage; g.b_slot = pl.b_slot; g.halo = pl.halo;
     {   // the epilogue stages two 128-pixel tiles in the operand rings when they fit
         const long long rings = (long long)pl.sa * pl.parts * pl.kg * (16 * pl.ma + 2) * mc::HALO_W * 16 + (long long)pl.sb * pl.b_slot;
-        // rows are staged in segments of NFE_MC_SEG_Q 16-column groups, one 128-row buffer per epilogue warp group that has an accumulator
+        // rows are staged in segments of SEG_Q16 16-column fp16 groups (128 bytes), one 128-row buffer per epilogue warp group that has an accumulator
         g.stage_ok = (pl.persist || pl.stage_bytes <= rings) ? 1 : 0;
     }
     g.tp = pl.tp;

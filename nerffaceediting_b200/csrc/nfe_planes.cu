@@ -145,28 +145,19 @@ __global__ void __launch_bounds__(256) to_channel_last_kernel(const float* __res
 // channel vector, i.e. one 128-byte channel-last texel, written as 8 float4 stores.  With NORMALIZE
 // the same registers also produce (x-mean)/(std+1e-8): the NCHW result (coalesced) and its channel-last
 // copy, so normalize_plane + both stagings cost one read of the planes instead of three.
-#ifndef NFE_STAGE_MIN_BLOCKS
-#define NFE_STAGE_MIN_BLOCKS 4
-#endif
-#ifndef NFE_STAGE_REVERSE
-#define NFE_STAGE_REVERSE 1   // c2 step 1.140 -> 1.136 ms on B200 (profiles/run_r01_stage_ab.sh)
-#endif
-#ifndef NFE_STAGE_STREAM
-#define NFE_STAGE_STREAM 1    // with the reverse walk: 1.134-1.136 ms
-#endif
+constexpr int STAGE_MIN_BLOCKS = 4;
 template <bool NORMALIZE>
-__global__ void __launch_bounds__(256, NFE_STAGE_MIN_BLOCKS) stage32_kernel(const float* __restrict__ planes, const float* __restrict__ mean,
+__global__ void __launch_bounds__(256, STAGE_MIN_BLOCKS) stage32_kernel(const float* __restrict__ planes, const float* __restrict__ mean,
                                                       const float* __restrict__ std_in, int64_t hw, int64_t groups_per_img, int64_t n_groups,
                                                       float* __restrict__ out_norm, float* __restrict__ out_norm_cl, float* __restrict__ out_raw_cl)
 {
     const int lane = threadIdx.x & 31;
     int64_t group = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (group >= n_groups) return;
-#if NFE_STAGE_REVERSE
     // normalize_plane runs right after plane_stats_kernel has streamed the same planes in ascending order: walking them in
     // DESCENDING order finds the last ~100 MB still in the 126 MB L2, and leaves item 0's staged copy hot for the field kernel
+    // (c2 step 1.140 -> 1.136 ms on B200, profiles/run_r01_stage_ab.sh)
     if constexpr (NORMALIZE) group = n_groups - 1 - group;
-#endif
     const int64_t img = group / groups_per_img;
     const int64_t px = (group % groups_per_img) * 32 + lane;
     const bool live = px < hw;
@@ -190,12 +181,9 @@ __global__ void __launch_bounds__(256, NFE_STAGE_MIN_BLOCKS) stage32_kernel(cons
         }
         if (live) {
             float* dn = out_norm + img * 32 * hw + px;
+            // the reference-layout copy is rarely read back: evict first (with the descending walk: c2 step 1.134-1.136 ms)
 #pragma unroll
-#if NFE_STAGE_STREAM
-            for (int c = 0; c < 32; ++c) __stcs(dn + (int64_t)c * hw, x[c]);     // the reference-layout copy is rarely read back: evict first
-#else
-            for (int c = 0; c < 32; ++c) dn[(int64_t)c * hw] = x[c];
-#endif
+            for (int c = 0; c < 32; ++c) __stcs(dn + (int64_t)c * hw, x[c]);
             float4* dst = reinterpret_cast<float4*>(out_norm_cl + (img * hw + px) * 32);
 #pragma unroll
             for (int q = 0; q < 8; ++q) dst[q] = make_float4(x[4 * q], x[4 * q + 1], x[4 * q + 2], x[4 * q + 3]);

@@ -12,7 +12,8 @@ namespace {
 struct Workspace {
     float* minmax;    // 2 floats (+pad)
     float* sigma_c; float* rec_c;   // densities (compact, for the weights / merge) and packed records {sigma,seg[15],rgb[32]}
-    float* w_c;       // coarse weights [T, s_c-1]
+    float* w_c;       // [T, s_c-1], not written: resample_kernel forms the coarse weights itself.  Its size stays in
+                      // nfe_render_workspace_bytes, which sets how ops.render_fwd chunks a large render (and so each chunk's Philox offset)
     float* depths_f;  // [T, s_f]
     float* sigma_f; float* rec_f;
     int64_t bytes;
@@ -126,20 +127,11 @@ NFE_EXPORT int nfe_render_fwd(const nfe_render_cfg* cfg, const nfe_mlp* net_a, c
     m.n_rays = rays; m.white_back = cfg->white_back;
     if (sf > 0) {
         // ---- coarse weights (renderer.py:118,340) and importance resampling (:120,342)
-        // One kernel: coarse compositing weights from the densities, then the inverse-CDF draw.  $NFE_SPLIT_COARSE=1 keeps the two
-        // launches (march_kernel<false> writing the weights, resample_kernel reading them back)
-        static const bool split = getenv("NFE_SPLIT_COARSE") != nullptr;
-        float* wc = weights_coarse_out ? weights_coarse_out : w.w_c;
-        if (split) {
-            m.depths1 = depths_coarse; m.sigma1 = w.sigma_c; m.s1 = sc; m.s2 = 0; m.cc = 0; m.cs = 0; m.weights = wc;
-            StageScope t(STAGE_MARCH_COARSE, stream);
-            if (int rc = launch_march(m, false, stream)) return rc;
-        }
+        // One kernel: coarse compositing weights from the densities, then the inverse-CDF draw
         float* df = depths_fine_out ? depths_fine_out : w.depths_f;
         ResampleArgs r = {};
         r.z_vals = depths_coarse; r.n_rays = rays; r.S = sc; r.s_f = sf; r.smooth = 1; r.eps = 1e-5f; r.sort_u = 1;
-        if (split) r.weights = wc;
-        else { r.sigma = w.sigma_c; r.weights_out = weights_coarse_out; }
+        r.sigma = w.sigma_c; r.weights_out = weights_coarse_out;
         r.u = cfg->stochastic ? nullptr : u_fine; r.u_per_ray = 0; r.seed = cfg->seed; r.offset = cfg->offset + 2; r.out = df;
         {
             StageScope t(STAGE_RESAMPLE, stream);
