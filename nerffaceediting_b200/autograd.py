@@ -18,12 +18,12 @@ Gradients reach the two plane tensors and the decoder parameters; sample positio
 are data and depths_fine is detached in the reference, renderer.py:198,211).
 """
 import ctypes
-import os
 
 import torch
 import torch.nn.functional as F
 
 from . import _lib, ops
+from .renderer import render_planes, run_model_planes
 
 MAX_ROWS = 1 << 22     # decoder-backward chunk (rows of [M,32] features) to bound the GEMM intermediates
 
@@ -54,10 +54,10 @@ class _FieldBackward:
     channel-last plane gradients, decoder-parameter gradients and (single-gather identity) the statistics gradients.
     Samples are either rays x depths (renderer forward) or explicit points (run_model)."""
 
-    def __init__(self, kind, seq_a, seq_b, norm_cl, denorm_cl, affine, box_warp, needs_param_grad, dev):
-        self.kind, self.seq_a, self.seq_b = kind, seq_a, seq_b
-        self.norm_cl, self.denorm_cl, self.affine, self.box_warp, self.dev = norm_cl, denorm_cl, affine, box_warp, dev
-        self.params = _decoder_params(seq_a, seq_b)
+    def __init__(self, plan, norm_cl, denorm_cl, box_warp, needs_param_grad, dev):
+        self.kind, self.seq_a, self.seq_b, self.affine = plan.kind, plan.seq_a, plan.seq_b, plan.affine
+        self.norm_cl, self.denorm_cl, self.box_warp, self.dev = norm_cl, denorm_cl, box_warp, dev
+        self.params = _decoder_params(plan.seq_a, plan.seq_b)
         self.live = [i for i, need in enumerate(needs_param_grad) if need]
         self.g_params = [torch.zeros_like(p) if i in self.live else None for i, p in enumerate(self.params)]
         any_cl = denorm_cl if denorm_cl is not None else norm_cl
@@ -65,11 +65,11 @@ class _FieldBackward:
         self.g_denorm_cl = torch.zeros_like(denorm_cl) if denorm_cl is not None else None
         self.g_norm_cl = torch.zeros_like(norm_cl) if norm_cl is not None else None
         self.g_scale = self.g_shift = None
-        if affine is not None:
-            self.g_scale, self.g_shift = torch.zeros_like(affine[0]), torch.zeros_like(affine[1])
+        if self.affine is not None:
+            self.g_scale, self.g_shift = torch.zeros_like(self.affine[0]), torch.zeros_like(self.affine[1])
         # one tcgen05 kernel per pass (csrc/nfe_field_bwd.cu, templated on the decoder kind); NFE_BWD_LIBRARY_GEMM=1 keeps the
         # cross-check path: the MLP backward on library GEMMs (torch.addmm) between two gather kernels
-        self.fused = affine is not None or os.environ.get("NFE_BWD_LIBRARY_GEMM", "0") != "1"
+        self.fused = not plan.library_gemm
         if self.fused:
             self.full = [g if g is not None else torch.zeros_like(p) for g, p in zip(self.g_params, self.params)]
 
@@ -159,30 +159,16 @@ class _FieldBackward:
         return g_norm, g_planes, g_scale, g_shift, self.g_params
 
 
-def _affine_of(scale_src, shift_src, eps):
-    if scale_src is None:
-        return None
-    k = scale_src.numel() // 96
-    return ((scale_src.detach().reshape(k, 96).float() + eps).contiguous(), shift_src.detach().reshape(k, 96).float().contiguous())
-
-
 class RenderFunction(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, state, norm_planes, planes, scale_src, shift_src, *params):
-        """state: dict(kind, seq_a, seq_b, cfg kwargs, rays, depths_coarse, u_fine[, affine_eps]).  params are the decoder
-        parameters, passed only so that autograd tracks them; the kernels read them from the modules.
-        scale_src / shift_src (or None): statistics with planes == norm_planes*(scale_src + affine_eps) + shift_src per
-        (item, channel) — the single-gather identity: `planes` is then never read and its gradient flows through them."""
-        kind = state["kind"]
-        affine = _affine_of(scale_src, shift_src, state.get("affine_eps", 0.0))
-        denorm_cl = ops.planes_channel_last(planes) if affine is None else None
-        norm_cl = ops.planes_channel_last(norm_planes) if kind == ops.DEC_DISENTANGLED else None
-        cfg = ops.make_cfg(kind, norm_cl if denorm_cl is None else denorm_cl, affine=affine, **state["cfg"])
-        o, d = state["rays"]
-        rgb, seg, depth, wsum, minmax, st = ops.render_fwd(cfg, state["seq_a"], state["seq_b"], norm_cl, denorm_cl, o, d, state["depths_coarse"],
-                                                          state["u_fine"], return_stages=True, keep_workspace=True)
-        ctx.state, ctx.cfg = state, cfg
-        ctx.affine = affine
+    def forward(ctx, plan, args, norm_planes, planes, scale_src, shift_src, *params):
+        """plan: renderer.field_plan's decision; args: renderer.render_planes' (origins, dirs, depths_coarse, u_fine, opts,
+        stochastic, seed, offset).  params are the decoder parameters, passed only so that autograd tracks them; the kernels
+        read them from the modules.  scale_src / shift_src: plan.sources or None — under the single-gather identity
+        `planes` is never read and its gradient flows through these statistics."""
+        cfg, norm_cl, denorm_cl, (rgb, seg, depth, wsum, minmax, st) = render_planes(plan, norm_planes, planes, *args, return_stages=True,
+                                                                                      keep_workspace=True)
+        ctx.plan, ctx.cfg, ctx.rays = plan, cfg, args[:3]
         ctx.stat_shapes = None if scale_src is None else (scale_src.shape, shift_src.shape)
         ctx.saved = (norm_cl, denorm_cl, st, minmax)
         ctx.plane_shapes = (None if norm_planes is None else norm_planes.shape, planes.shape)
@@ -193,15 +179,13 @@ class RenderFunction(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, *grads):
-        state, cfg = ctx.state, ctx.cfg
-        kind, seq_a, seq_b = state["kind"], state["seq_a"], state["seq_b"]
+        cfg = ctx.cfg
         norm_cl, denorm_cl, st, minmax = ctx.saved
-        has_seg = kind != ops.DEC_OSG
-        if has_seg:
+        if ctx.plan.kind != ops.DEC_OSG:
             g_rgb, g_seg, g_depth, g_wsum = grads[0], grads[1], grads[2], grads[3]
         else:
             g_rgb, g_seg, g_depth, g_wsum = grads[0], None, grads[1], grads[2]
-        o, d = state["rays"]
+        o, d, depths_coarse = ctx.rays
         n, r, _ = o.shape
         dev = o.device
         s_c, s_f = cfg.s_c, cfg.s_f
@@ -212,7 +196,7 @@ class RenderFunction(torch.autograd.Function):
             return None if t is None else t.contiguous().float()
         g_rgb = f32(g_rgb) if g_rgb is not None else torch.zeros((n, r, 32), device=dev)
         g_seg, g_depth, g_wsum = f32(g_seg), f32(g_depth), f32(g_wsum)
-        dc = state["depths_coarse"].reshape(n, r, s_c).contiguous()
+        dc = depths_coarse.reshape(n, r, s_c).contiguous()
         df = st["depths_fine"].reshape(n, r, s_f).contiguous() if s_f else None
         g_rec_c = torch.empty((n * r, s_c, 48), device=dev)
         g_rec_f = torch.empty((n * r, s_f, 48), device=dev) if s_f else None
@@ -223,16 +207,15 @@ class RenderFunction(torch.autograd.Function):
                                              n * r, cfg.seg_dim, cfg.white_back, P(g_rgb), P(g_seg), P(g_depth), P(g_wsum), P(minmax),
                                              P(g_rec_c), P(g_rec_f), stream), "nfe_composite_bwd")
             # 2-4. gather + decoder backward of both passes
-            fb = _FieldBackward(kind, seq_a, seq_b, norm_cl, denorm_cl, ctx.affine, cfg.box_warp, ctx.needs_input_grad[5:], dev)
+            fb = _FieldBackward(ctx.plan, norm_cl, denorm_cl, cfg.box_warp, ctx.needs_input_grad[6:], dev)
             for depths, s, rec, g_rec in ((dc, s_c, st["rec_c"], g_rec_c), (df, s_f, st.get("rec_f"), g_rec_f)):
                 if s:
                     fb.run_pass(n, rec, g_rec, rays=(o, d, depths))
             # 5. back to the reference layout
             norm_shape, plane_shape = ctx.plane_shapes
-            stat = ctx.stat_shapes
-            g_norm, g_planes, g_scale, g_shift, g_params = fb.finish(norm_shape, plane_shape, ctx.needs_input_grad[1], ctx.needs_input_grad[2], stat,
-                                                                     ctx.needs_input_grad[3], ctx.needs_input_grad[4])
-        return (None, g_norm, g_planes, g_scale, g_shift) + tuple(g_params)
+            g_norm, g_planes, g_scale, g_shift, g_params = fb.finish(norm_shape, plane_shape, *ctx.needs_input_grad[2:4], ctx.stat_shapes,
+                                                                     *ctx.needs_input_grad[4:6])
+        return (None, None, g_norm, g_planes, g_scale, g_shift) + tuple(g_params)
 
 
 class RunModelFunction(torch.autograd.Function):
@@ -241,28 +224,19 @@ class RunModelFunction(torch.autograd.Function):
     the statistics, under the single-gather identity) and the decoder parameters; the sample coordinates carry none."""
 
     @staticmethod
-    def forward(ctx, state, norm_planes, planes, scale_src, shift_src, *params):
-        kind = state["kind"]
-        coords = state["coords"]
-        sigma_only = state["sigma_only"]
-        affine = _affine_of(scale_src, shift_src, state.get("affine_eps", 0.0))
-        geo_only = sigma_only and kind == ops.DEC_DISENTANGLED and state["cfg"]["precision"] != ops.PRECISIONS['fp32']
-        norm_cl = ops.planes_channel_last(norm_planes) if kind == ops.DEC_DISENTANGLED else None
-        denorm_cl = ops.planes_channel_last(planes) if affine is None else None
-        cfg = ops.make_cfg(kind, norm_cl if denorm_cl is None else denorm_cl, 2, 0, affine=affine, **state["cfg"])
-        out = ops.run_model_fwd(cfg, state["seq_a"], state["seq_b"], norm_cl, None if (geo_only and affine is not None) else denorm_cl, coords,
-                                sigma_only=sigma_only)
-        ctx.state, ctx.affine, ctx.box_warp = state, affine, cfg.box_warp
+    def forward(ctx, plan, args, norm_planes, planes, scale_src, shift_src, *params):
+        """As RenderFunction.forward; args: renderer.run_model_planes' (coords, opts, seed, offset, sigma_only)."""
+        cfg, norm_cl, denorm_cl, out = run_model_planes(plan, norm_planes, planes, *args)
+        ctx.plan, ctx.coords, ctx.box_warp = plan, args[0], cfg.box_warp
         ctx.stat_shapes = None if scale_src is None else (scale_src.shape, shift_src.shape)
-        ctx.saved = (norm_cl, denorm_cl, None if sigma_only else out["rgb"])
+        ctx.saved = (norm_cl, denorm_cl, out.get("rgb"))
         ctx.plane_shapes = (None if norm_planes is None else norm_planes.shape, planes.shape)
-        ctx.keys = ("sigma",) if sigma_only else tuple(k for k in ("rgb", "sigma", "seg") if k in out)
+        ctx.keys = tuple(k for k in ("rgb", "sigma", "seg") if k in out)
         return tuple(out[k] for k in ctx.keys)
 
     @staticmethod
     def backward(ctx, *grads):
-        state = ctx.state
-        kind, seq_a, seq_b, coords = state["kind"], state["seq_a"], state["seq_b"], state["coords"]
+        coords = ctx.coords
         norm_cl, denorm_cl, rgb = ctx.saved
         n, m, _ = coords.shape
         dev = coords.device
@@ -279,12 +253,12 @@ class RunModelFunction(torch.autograd.Function):
         if g.get("rgb") is not None:
             g_rec[:, 16:48] = g["rgb"].reshape(n * m, 32)
         with torch.cuda.device(dev):
-            fb = _FieldBackward(kind, seq_a, seq_b, norm_cl, denorm_cl, ctx.affine, ctx.box_warp, ctx.needs_input_grad[5:], dev)
+            fb = _FieldBackward(ctx.plan, norm_cl, denorm_cl, ctx.box_warp, ctx.needs_input_grad[6:], dev)
             fb.run_pass(n, rec, g_rec, coords=coords)
             norm_shape, plane_shape = ctx.plane_shapes
-            g_norm, g_planes, g_scale, g_shift, g_params = fb.finish(norm_shape, plane_shape, ctx.needs_input_grad[1], ctx.needs_input_grad[2],
-                                                                     ctx.stat_shapes, ctx.needs_input_grad[3], ctx.needs_input_grad[4])
-        return (None, g_norm, g_planes, g_scale, g_shift) + tuple(g_params)
+            g_norm, g_planes, g_scale, g_shift, g_params = fb.finish(norm_shape, plane_shape, *ctx.needs_input_grad[2:4], ctx.stat_shapes,
+                                                                     *ctx.needs_input_grad[4:6])
+        return (None, None, g_norm, g_planes, g_scale, g_shift) + tuple(g_params)
 
 
 class NormalizeFunction(torch.autograd.Function):

@@ -267,6 +267,34 @@ int check_decoder_dims(int kind, const nfe_mlp* net_a, const nfe_mlp* net_b, con
     return 0;
 }
 
+int field_planes(const nfe_render_cfg* cfg, const float* planes_norm_cl, const float* planes_denorm_cl, int plane_batch, int n,
+                 int64_t pass_samples, bool sigma_only, const char* who, FieldArgs& f)
+{
+    NFE_REQUIRE(cfg->channels == FEAT, "%s: planes must have %d channels (got %d)", who, FEAT, cfg->channels);
+    NFE_REQUIRE(cfg->height >= 1 && cfg->width >= 1, "%s: bad plane size", who);
+    NFE_REQUIRE(cfg->box_warp != 0.0f, "%s: box_warp must be non-zero", who);
+    NFE_REQUIRE(cfg->precision >= NFE_PREC_FP32 && cfg->precision <= NFE_PREC_BF16, "%s: unknown precision mode %d", who, cfg->precision);
+    NFE_REQUIRE(cfg->seg_dim == (cfg->kind == NFE_DEC_OSG ? 0 : 15), "%s: seg_dim %d unsupported for decoder kind %d", who, cfg->seg_dim, cfg->kind);
+    const bool disentangled_tc = cfg->kind == NFE_DEC_DISENTANGLED && cfg->precision != NFE_PREC_FP32;
+    // single-gather identity (cfg->affine_*): the de-normalised planes are norm*scale + shift and are not read
+    const bool affine = cfg->affine_scale && cfg->affine_shift && disentangled_tc;
+    // a density-only query with the disentangled decoder on the tensor cores reads the normalised planes only
+    const bool geo_only = sigma_only && disentangled_tc;
+    NFE_REQUIRE(!cfg->affine_scale || cfg->affine_items == 1 || cfg->affine_items == n, "%s: affine statistics for %d items, batch is %d", who,
+                cfg->affine_items, n);
+    // the field kernel keeps the statistics of two batch items per 128-sample tile: an item must span at least one tile in each pass
+    NFE_REQUIRE(!affine || pass_samples >= 128, "%s: the single-gather identity needs at least 128 samples per item and pass (%lld)", who,
+                (long long)pass_samples);
+    NFE_REQUIRE(planes_denorm_cl || affine || geo_only, "%s: null pointer to the de-normalised planes", who);
+    NFE_REQUIRE(cfg->kind != NFE_DEC_DISENTANGLED || planes_norm_cl, "%s: the disentangled decoder needs the normalised planes", who);
+    NFE_REQUIRE(plane_batch == n || plane_batch == 1, "%s: plane batch %d does not match batch %d", who, plane_batch, n);
+    f.set_norm = planes_norm_cl; f.set_denorm = planes_denorm_cl; f.plane_batch = plane_batch; f.H = cfg->height; f.W = cfg->width;
+    f.scale = (float)(2.0 / (double)cfg->box_warp);
+    if (affine) { f.affine_scale = cfg->affine_scale; f.affine_shift = cfg->affine_shift; f.affine_items = cfg->affine_items; }
+    f.sigma_only = sigma_only;
+    return 0;
+}
+
 int launch_field(int kind, int precision, const FieldArgs& a, const nfe_mlp* net_a, const nfe_mlp* net_b, cudaStream_t stream)
 {
     if (a.total <= 0) return 0;
@@ -351,28 +379,15 @@ NFE_EXPORT int nfe_run_model_fwd(const nfe_render_cfg* cfg, const nfe_mlp* net_a
     (void)workspace; (void)workspace_bytes;
     NFE_REQUIRE(cfg, "nfe_run_model_fwd: null cfg");
     if (int rc = check_decoder_dims(cfg->kind, net_a, net_b, "nfe_run_model_fwd")) return rc;
-    NFE_REQUIRE(cfg->channels == FEAT, "nfe_run_model_fwd: planes must have %d channels (got %d)", FEAT, cfg->channels);
     if ((int64_t)n * m == 0) return 0;
     const bool sigma_only = cfg->sigma_only != 0;
-    const bool geo_only = sigma_only && cfg->kind == NFE_DEC_DISENTANGLED && cfg->precision != NFE_PREC_FP32;
-    // single-gather identity (cfg->affine_*): the de-normalised planes are norm*scale + shift and are not read
-    const bool affine = cfg->affine_scale && cfg->affine_shift && cfg->kind == NFE_DEC_DISENTANGLED && cfg->precision != NFE_PREC_FP32;
-    NFE_REQUIRE(!cfg->affine_scale || cfg->affine_items == 1 || cfg->affine_items == n, "nfe_run_model_fwd: affine statistics for %d items, batch is %d",
-                cfg->affine_items, n);
-    NFE_REQUIRE((planes_denorm_cl || geo_only || affine) && coords && sigma && (rgb || sigma_only), "nfe_run_model_fwd: null pointer");
-    NFE_REQUIRE(!affine || m >= 128, "nfe_run_model_fwd: the single-gather identity needs at least 128 points per item (%lld)", (long long)m);
-    NFE_REQUIRE(cfg->kind != NFE_DEC_DISENTANGLED || planes_norm_cl, "nfe_run_model_fwd: the disentangled decoder needs the normalised planes");
-    NFE_REQUIRE(cfg->kind == NFE_DEC_OSG || seg || sigma_only, "nfe_run_model_fwd: seg output missing");
-    NFE_REQUIRE(plane_batch == n || plane_batch == 1, "nfe_run_model_fwd: plane batch %d does not match point batch %d", plane_batch, n);
-    NFE_REQUIRE(cfg->precision >= NFE_PREC_FP32 && cfg->precision <= NFE_PREC_BF16, "nfe_run_model_fwd: unknown precision mode %d", cfg->precision);
     FieldArgs a = {};
-    a.set_norm = planes_norm_cl; a.set_denorm = planes_denorm_cl; a.plane_batch = plane_batch; a.H = cfg->height; a.W = cfg->width;
-    a.scale = (float)(2.0 / (double)cfg->box_warp);
-    if (affine) { a.affine_scale = cfg->affine_scale; a.affine_shift = cfg->affine_shift; a.affine_items = cfg->affine_items; }
+    if (int rc = field_planes(cfg, planes_norm_cl, planes_denorm_cl, plane_batch, n, m, sigma_only, "nfe_run_model_fwd", a)) return rc;
+    NFE_REQUIRE(coords && sigma && (rgb || sigma_only), "nfe_run_model_fwd: null pointer");
+    NFE_REQUIRE(cfg->kind == NFE_DEC_OSG || seg || sigma_only, "nfe_run_model_fwd: seg output missing");
     a.coords = coords; a.m = m; a.total = (int64_t)n * m; a.s_per_ray = 1;
     a.sigma = sigma; a.rgb = rgb; a.seg = seg;
     a.density_noise = cfg->density_noise; a.seed = cfg->seed; a.offset = cfg->offset;
-    a.sigma_only = sigma_only;
     StageScope t(STAGE_RUN_MODEL, as_stream(stream));
     return launch_field(cfg->kind, cfg->precision, a, net_a, net_b, as_stream(stream));
 }

@@ -45,22 +45,6 @@ Workspace carve(const nfe_render_cfg* cfg, int64_t rays, void* base)
     return w;
 }
 
-int check_cfg(const nfe_render_cfg* cfg, const char* who)
-{
-    NFE_REQUIRE(cfg, "%s: null cfg", who);
-    NFE_REQUIRE(cfg->channels == 32, "%s: planes must have 32 channels (got %d)", who, cfg->channels);
-    NFE_REQUIRE(cfg->height >= 1 && cfg->width >= 1, "%s: bad plane size", who);
-    NFE_REQUIRE(cfg->s_c >= 2, "%s: depth_resolution must be >= 2 (got %d)", who, cfg->s_c);
-    NFE_REQUIRE(cfg->s_f >= 0, "%s: depth_resolution_importance must be >= 0", who);
-    NFE_REQUIRE(cfg->s_f == 0 || cfg->s_c >= 4, "%s: importance sampling needs depth_resolution >= 4", who);
-    NFE_REQUIRE(cfg->s_c + cfg->s_f <= MAX_S, "%s: %d+%d samples per ray exceed %d", who, cfg->s_c, cfg->s_f, MAX_S);
-    NFE_REQUIRE(cfg->color_dim == 32, "%s: decoder_output_dim must be 32 (got %d)", who, cfg->color_dim);
-    NFE_REQUIRE(cfg->seg_dim == (cfg->kind == NFE_DEC_OSG ? 0 : 15), "%s: seg_dim %d unsupported for decoder kind %d", who, cfg->seg_dim, cfg->kind);
-    NFE_REQUIRE(cfg->box_warp != 0.0f, "%s: box_warp must be non-zero", who);
-    NFE_REQUIRE(cfg->precision >= NFE_PREC_FP32 && cfg->precision <= NFE_PREC_BF16, "%s: unknown precision mode %d", who, cfg->precision);
-    return 0;
-}
-
 }  // namespace
 
 NFE_EXPORT int64_t nfe_render_workspace_bytes(const nfe_render_cfg* cfg, int n, int64_t n_rays)
@@ -84,35 +68,29 @@ NFE_EXPORT int nfe_render_fwd(const nfe_render_cfg* cfg, const nfe_mlp* net_a, c
                               float* minmax_out, int finish_depth, float* depths_fine_out, float* weights_coarse_out, void* workspace,
                               int64_t workspace_bytes, nfe_stream_t stream_)
 {
-    if (int rc = check_cfg(cfg, "nfe_render_fwd")) return rc;
+    NFE_REQUIRE(cfg, "nfe_render_fwd: null cfg");
+    NFE_REQUIRE(cfg->s_c >= 2, "nfe_render_fwd: depth_resolution must be >= 2 (got %d)", cfg->s_c);
+    NFE_REQUIRE(cfg->s_f >= 0, "nfe_render_fwd: depth_resolution_importance must be >= 0");
+    NFE_REQUIRE(cfg->s_f == 0 || cfg->s_c >= 4, "nfe_render_fwd: importance sampling needs depth_resolution >= 4");
+    NFE_REQUIRE(cfg->s_c + cfg->s_f <= MAX_S, "nfe_render_fwd: %d+%d samples per ray exceed %d", cfg->s_c, cfg->s_f, MAX_S);
+    NFE_REQUIRE(cfg->color_dim == 32, "nfe_render_fwd: decoder_output_dim must be 32 (got %d)", cfg->color_dim);
     if (int rc = check_decoder_dims(cfg->kind, net_a, net_b, "nfe_render_fwd")) return rc;
-    if ((int64_t)n * n_rays == 0) return 0;  // empty tensors carry null pointers
-    const bool affine = cfg->affine_scale && cfg->affine_shift && cfg->kind == NFE_DEC_DISENTANGLED && cfg->precision != NFE_PREC_FP32;
-    NFE_REQUIRE(!cfg->affine_scale || (cfg->affine_items == 1 || cfg->affine_items == n), "nfe_render_fwd: affine statistics for %d items, batch is %d",
-                cfg->affine_items, n);
-    NFE_REQUIRE((planes_denorm_cl || affine) && origins && dirs && depths_coarse && rgb && depth && wsum, "nfe_render_fwd: null pointer");
-    // the field kernel keeps the statistics of two batch items per 128-sample tile: an item must span at least one tile in each pass
-    NFE_REQUIRE(!affine || (n_rays * cfg->s_c >= 128 && (cfg->s_f == 0 || n_rays * cfg->s_f >= 128)),
-                "nfe_render_fwd: the single-gather identity needs at least 128 samples per item and pass (%lld rays x %d / %d)", (long long)n_rays,
-                cfg->s_c, cfg->s_f);
-    NFE_REQUIRE(cfg->kind != NFE_DEC_DISENTANGLED || planes_norm_cl, "nfe_render_fwd: the disentangled decoder needs the normalised planes");
-    NFE_REQUIRE(cfg->seg_dim == 0 || seg, "nfe_render_fwd: seg output missing");
-    NFE_REQUIRE(plane_batch == n || plane_batch == 1, "nfe_render_fwd: plane batch %d does not match ray batch %d", plane_batch, n);
-    NFE_REQUIRE(cfg->s_f == 0 || cfg->stochastic || u_fine, "nfe_render_fwd: parity mode needs the u_fine table");
     const int64_t rays = (int64_t)n * n_rays;
-    if (rays == 0) return 0;
+    if (rays == 0) return 0;  // empty tensors carry null pointers
+    const int sc = cfg->s_c, sf = cfg->s_f;
+    const int64_t pass_samples = n_rays * (sf > 0 && sf < sc ? sf : sc);
+    FieldArgs f = {};
+    if (int rc = field_planes(cfg, planes_norm_cl, planes_denorm_cl, plane_batch, n, pass_samples, false, "nfe_render_fwd", f)) return rc;
+    NFE_REQUIRE(origins && dirs && depths_coarse && rgb && depth && wsum, "nfe_render_fwd: null pointer");
+    NFE_REQUIRE(cfg->seg_dim == 0 || seg, "nfe_render_fwd: seg output missing");
+    NFE_REQUIRE(cfg->s_f == 0 || cfg->stochastic || u_fine, "nfe_render_fwd: parity mode needs the u_fine table");
     NFE_REQUIRE(workspace, "nfe_render_fwd: null workspace");
     const Workspace w = carve(cfg, rays, workspace);
     NFE_REQUIRE(workspace_bytes >= w.bytes, "nfe_render_fwd: workspace too small (%lld < %lld bytes)", (long long)workspace_bytes, (long long)w.bytes);
     cudaStream_t stream = as_stream(stream_);
-    const int sc = cfg->s_c, sf = cfg->s_f;
     float* minmax = minmax_out ? minmax_out : w.minmax;
 
     // ---- coarse pass (renderer.py:104-113,325-336)
-    FieldArgs f = {};
-    f.set_norm = planes_norm_cl; f.set_denorm = planes_denorm_cl; f.plane_batch = plane_batch; f.H = cfg->height; f.W = cfg->width;
-    if (affine) { f.affine_scale = cfg->affine_scale; f.affine_shift = cfg->affine_shift; f.affine_items = cfg->affine_items; }
-    f.scale = (float)(2.0 / (double)cfg->box_warp);
     f.origins = origins; f.dirs = dirs; f.depths = depths_coarse; f.s_per_ray = sc;
     f.m = n_rays * sc; f.total = rays * sc;
     f.sigma = w.sigma_c; f.rec = w.rec_c;

@@ -29,12 +29,102 @@ Instances hold no state of their own beyond the reference's attributes, so objec
 reference checkpoints (which skip __init__, SURVEY.md §7.9) work.
 """
 import os
+from typing import NamedTuple
 
 import torch
 import torch.nn as nn
 
 from . import math_utils, ops
 from .ray_marcher import MipRayMarcher2, SegMipRayMarcher2
+
+
+class FieldPlan(NamedTuple):
+    """How the fused forward of one render or run_model call reads the tri-planes (made by field_plan)."""
+    kind: int
+    seq_a: object
+    seq_b: object           # None for the OSG decoder
+    precision: int
+    geo_only: bool          # density-only query, disentangled decoder on the tensor cores: the appearance net and its planes are skipped
+    affine: object          # (scale [K,96], shift [K,96]) under the single-gather identity, else None
+    sources: object         # training under the identity: (scale_src, shift_src), the autograd inputs of the affine pair, else None
+    stage_norm: bool        # which plane sets are staged channel-last
+    stage_denorm: bool
+    library_gemm: bool      # NFE_BWD_LIBRARY_GEMM=1: the backward runs the decoder MLPs on library GEMMs (autograd._FieldBackward)
+    path: object            # (what, path) for ops.note_path, or None
+
+
+def field_plan(what, desc, norm_planes, planes, opts, batch, per_item, grad, sigma_only=False):
+    """Decide the fused forward of one call: what = 'render' (per_item rays per batch item) or 'run_model' (per_item points),
+    desc = ops.describe_decoder(decoder), grad = whether the call is differentiable.  It reads the options, the environment
+    and the plane registries and calls no kernel, so it runs on CPU tensors as well."""
+    kind, seq_a, seq_b = desc
+    precision = ops.precision_of(opts)
+    disentangled_tc = kind == ops.DEC_DISENTANGLED and precision != ops.PRECISIONS['fp32']
+    geo_only = sigma_only and disentangled_tc
+    library_gemm = os.environ.get("NFE_BWD_LIBRARY_GEMM", "0") == "1"
+    if what == "render":
+        s_c, s_f = opts['depth_resolution'], opts['depth_resolution_importance']
+        per_item *= min(s_c, s_f if s_f > 0 else s_c)
+    # The field kernel keeps the statistics of at most two batch items per 128-sample tile, so the single-gather identity needs
+    # every item to hold at least one tile's worth of samples in each pass (always true for renders; tiny point queries simply
+    # read both plane sets).
+    single = disentangled_tc and opts.get('nfe_single_gather', True) and per_item >= 128
+    affine = sources = None
+    if not grad:
+        # planes known to be norm*scale + shift per channel (normalize_plane / denormalize_plane made them): gather the
+        # normalised planes only and rebuild the de-normalised features from the statistics
+        if single and not geo_only:
+            affine = ops.provenance(norm_planes, planes)
+        path = (what, "single-gather" if (affine is not None or geo_only) else ("two-gather" if kind == ops.DEC_DISENTANGLED else "one-set"))
+    else:
+        # In training the identity replaces the gradient into `planes` by gradients into the normalised planes and the
+        # statistics `planes` is tied to (normalize_plane: planes is their root; denormalize_plane: planes is their product),
+        # which is only the same thing while the autograd graph still has the shape it had when the pair was made: `planes`
+        # must carry grad and `norm_planes` must be in the state it was registered in.  A pair with one branch detached
+        # afterwards (renderer(norm.detach(), planes), renderer(norm, planes.detach())) takes the two-gather backward, which
+        # honours the detach like the reference does.  The library-GEMM cross-check of the backward reads both plane sets.
+        src = ops.provenance_sources(norm_planes, planes) if (single and not library_gemm) else None
+        if (src is not None and src[0].numel() == src[2].numel() and src[0].numel() in (96, 96 * batch)
+                and planes.requires_grad and bool(norm_planes.requires_grad) == src[3]):
+            scale_src, eps, shift_src, _ = src
+            k = scale_src.numel() // 96
+            affine = ((scale_src.detach().reshape(k, 96).float() + eps).contiguous(), shift_src.detach().reshape(k, 96).float().contiguous())
+            sources = (scale_src, shift_src)
+        path = (what, "training-single-gather" if sources else "training") if what == "render" else None
+    # a differentiable run_model stages the raw planes even when geometry-only: its backward returns their gradient in that shape
+    return FieldPlan(kind, seq_a, seq_b, precision, geo_only, affine, sources, kind == ops.DEC_DISENTANGLED,
+                     affine is None and not (geo_only and not grad), library_gemm, path)
+
+
+def _stage(plan, norm_planes, planes, cache):
+    """Channel-last staging of the plane sets `plan` reads: (norm_cl, denorm_cl), None for a set that is not read."""
+    norm_cl = ops.planes_channel_last(norm_planes, cache) if plan.stage_norm else None
+    denorm_cl = ops.planes_channel_last(planes, cache) if plan.stage_denorm else None
+    return norm_cl, denorm_cl
+
+
+def render_planes(plan, norm_planes, planes, origins, dirs, depths_coarse, u_fine, opts, stochastic, seed, offset, cache=False,
+                  image_layout=False, **taps):
+    """Fused render forward of inference and of autograd.RenderFunction: stage, build the cfg, ops.render_fwd (taps are its
+    finish_depth / return_stages / keep_workspace).  Returns (cfg, norm_cl, denorm_cl, render_fwd's outputs)."""
+    norm_cl, denorm_cl = _stage(plan, norm_planes, planes, cache)
+    planes_cl = norm_cl if denorm_cl is None else denorm_cl
+    if planes_cl.shape[0] not in (1, origins.shape[0]):
+        raise RuntimeError(f"planes batch {planes_cl.shape[0]} does not match ray batch {origins.shape[0]}")
+    cfg = ops.make_cfg(plan.kind, planes_cl, opts['depth_resolution'], opts['depth_resolution_importance'], opts['box_warp'],
+                       opts.get('white_back', False), opts.get('density_noise', 0) or 0.0, stochastic=stochastic, seed=seed, offset=offset,
+                       precision=plan.precision, affine=plan.affine)
+    cfg.image_layout = int(image_layout)
+    return cfg, norm_cl, denorm_cl, ops.render_fwd(cfg, plan.seq_a, plan.seq_b, norm_cl, denorm_cl, origins, dirs, depths_coarse, u_fine, **taps)
+
+
+def run_model_planes(plan, norm_planes, planes, coords, opts, seed, offset, sigma_only, cache=False):
+    """Fused run_model forward of inference and of autograd.RunModelFunction: stage, build the cfg, ops.run_model_fwd.
+    Returns (cfg, norm_cl, denorm_cl, run_model_fwd's outputs)."""
+    norm_cl, denorm_cl = _stage(plan, norm_planes, planes, cache)
+    cfg = ops.make_cfg(plan.kind, norm_cl if denorm_cl is None else denorm_cl, 2, 0, opts['box_warp'], density_noise=opts.get('density_noise', 0) or 0.0,
+                       seed=seed, offset=offset, precision=plan.precision, affine=plan.affine)
+    return cfg, norm_cl, denorm_cl, ops.run_model_fwd(cfg, plan.seq_a, plan.seq_b, norm_cl, denorm_cl, coords, sigma_only=sigma_only)
 
 
 def generate_planes():
@@ -154,107 +244,37 @@ class ImportanceRenderer(torch.nn.Module):
             if defer_clamp:
                 raise NotImplementedError("a ray-sharded render needs one of the reference's decoders (fused path)")
             return self._render_staged(norm_planes, planes, decoder, ray_origins, ray_directions, opts, deterministic)
-        kind, seq_a, seq_b = desc
-        if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (norm_planes, planes, *decoder.parameters())):
-            if defer_clamp:
-                raise NotImplementedError("the ray-sharded render is inference-only")
-            return self._render_training(kind, seq_a, seq_b, norm_planes, planes, ray_origins, ray_directions, opts, deterministic)
-        cache = bool(opts.get('nfe_cache_planes', False))
-        precision = ops.precision_of(opts)
-        affine = None
-        if (kind == ops.DEC_DISENTANGLED and precision != ops.PRECISIONS['fp32'] and opts.get('nfe_single_gather', True)
-                and self._single_gather_fits(ray_origins.shape[1], opts)):
-            # planes known to be norm*scale + shift per channel (normalize_plane / denormalize_plane made them):
-            # gather the normalised planes only and rebuild the de-normalised features from the statistics
-            affine = ops.provenance(norm_planes, planes)
-        norm_cl = ops.planes_channel_last(norm_planes, cache) if kind == ops.DEC_DISENTANGLED else None
-        denorm_cl = ops.planes_channel_last(planes, cache) if affine is None else None
-        ops.note_path("render", "single-gather" if affine is not None else ("two-gather" if kind == ops.DEC_DISENTANGLED else "one-set"))
-        plane_batch = (norm_cl if denorm_cl is None else denorm_cl).shape[0]
-        if plane_batch not in (1, ray_origins.shape[0]):
-            raise RuntimeError(f"planes batch {plane_batch} does not match ray batch {ray_origins.shape[0]}")
+        grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (norm_planes, planes, *decoder.parameters()))
+        if grad and defer_clamp:
+            raise NotImplementedError("the ray-sharded render is inference-only")
+        n, r, _ = ray_origins.shape
+        plan = field_plan("render", desc, norm_planes, planes, opts, n, r, grad)
+        ops.note_path(*plan.path)
+        image = bool(opts.get('nfe_image_layout', False)) and not defer_clamp and not grad
+        side = int(round(r ** 0.5))
+        if image and side * side != r:
+            raise RuntimeError("nfe_image_layout needs a square ray grid (RaySampler's res*res rays)")
         depths_coarse, seed, offset = self._coarse_depths(ray_origins, ray_directions, opts, deterministic)
         s_f = opts['depth_resolution_importance']
-        cfg = ops.make_cfg(kind, norm_cl if denorm_cl is None else denorm_cl, opts['depth_resolution'], s_f, opts['box_warp'],
-                           opts.get('white_back', False), opts.get('density_noise', 0) or 0.0, stochastic=not deterministic, seed=seed,
-                           offset=offset, precision=precision, affine=affine)
-        if opts.get('nfe_image_layout', False) and not defer_clamp:
-            side = int(round(ray_origins.shape[1] ** 0.5))
-            if side * side != ray_origins.shape[1]:
-                raise RuntimeError("nfe_image_layout needs a square ray grid (RaySampler's res*res rays)")
-            cfg.image_layout = 1
         u_fine = ops.linspace_table(0, 1, s_f, ray_origins.device) if (s_f > 0 and deterministic) else None
-        rgb, seg, depth, wsum, minmax = ops.render_fwd(cfg, seq_a, seq_b, norm_cl, denorm_cl, ray_origins, ray_directions,
-                                                       depths_coarse, u_fine, finish_depth=not defer_clamp)
+        if grad:
+            # differentiable forward (BASELINE config 4): the same fused kernels, workspace kept for autograd.RenderFunction's
+            # backward; gradients flow to the plane tensors (or the statistics, under the single-gather identity) and the decoder
+            from .autograd import RenderFunction, _decoder_params
+            args = (ray_origins.detach().float().contiguous(), ray_directions.detach().float().contiguous(), depths_coarse, u_fine, opts,
+                    not deterministic, seed, offset)
+            out = RenderFunction.apply(plan, args, norm_planes if plan.stage_norm else None, planes, *(plan.sources or (None, None)),
+                                       *_decoder_params(plan.seq_a, plan.seq_b))
+            return (out[0], None, out[1], out[2]) if plan.kind == ops.DEC_OSG else out[:4]
+        _, _, _, (rgb, seg, depth, wsum, minmax) = render_planes(
+            plan, norm_planes, planes, ray_origins, ray_directions, depths_coarse, u_fine, opts, not deterministic, seed, offset,
+            cache=bool(opts.get('nfe_cache_planes', False)), image_layout=image, finish_depth=not defer_clamp)
         if defer_clamp:
             return rgb, seg, depth, wsum, minmax
-        if cfg.image_layout:
-            side = int(round(ray_origins.shape[1] ** 0.5))
-            n = ray_origins.shape[0]
+        if image:
             return (rgb.view(n, 32, side, side), None if seg is None else seg.view(n, seg.shape[1], side, side),
                     depth.view(n, 1, side, side), wsum)
         return rgb, seg, depth, wsum
-
-    @staticmethod
-    def _single_gather_fits(samples_axis, opts=None):
-        """The field kernel keeps the statistics of at most two batch items per 128-sample tile, so the single-gather identity
-        needs every item to hold at least one tile's worth of samples in each pass (always true for renders; tiny point
-        queries simply read both plane sets)."""
-        if opts is None:
-            return samples_axis >= 128
-        s_f = opts['depth_resolution_importance']
-        return samples_axis * min(opts['depth_resolution'], s_f if s_f > 0 else opts['depth_resolution']) >= 128
-
-    def _render_training(self, kind, seq_a, seq_b, norm_planes, planes, ray_origins, ray_directions, opts, deterministic):
-        """Differentiable forward (BASELINE config 4): same fused kernels, workspace kept for the backward
-        (autograd.RenderFunction).  Gradients flow to the plane tensors and the decoder parameters."""
-        from .autograd import RenderFunction
-        with torch.no_grad():
-            depths_coarse, seed, offset = self._coarse_depths(ray_origins, ray_directions, opts, deterministic)
-        s_f = opts['depth_resolution_importance']
-        state = {
-            "kind": kind, "seq_a": seq_a, "seq_b": seq_b,
-            "cfg": dict(s_c=opts['depth_resolution'], s_f=s_f, box_warp=opts['box_warp'], white_back=opts.get('white_back', False),
-                        density_noise=opts.get('density_noise', 0) or 0.0, stochastic=not deterministic, seed=seed, offset=offset,
-                        precision=ops.precision_of(opts)),
-            "rays": (ray_origins.detach().float().contiguous(), ray_directions.detach().float().contiguous()),
-            "depths_coarse": depths_coarse,
-            "u_fine": ops.linspace_table(0, 1, s_f, ray_origins.device) if (s_f > 0 and deterministic) else None,
-        }
-        params = [p for seq in (seq_a, seq_b) if seq is not None for p in (seq[0].weight, seq[0].bias, seq[2].weight, seq[2].bias)]
-        # single-gather identity in training: planes known to be norm*scale + shift are never read; their gradient goes
-        # through the statistics instead (autograd.RenderFunction, csrc/nfe_field_bwd.cu AFFINE)
-        scale_src = shift_src = None
-        if (kind == ops.DEC_DISENTANGLED and state["cfg"]["precision"] != ops.PRECISIONS['fp32'] and opts.get('nfe_single_gather', True)
-                and self._single_gather_fits(ray_origins.shape[1], opts)):
-            scale_src, shift_src = self._affine_sources(norm_planes, planes, ray_origins.shape[0], state)
-        ops.note_path("render", "training-single-gather" if scale_src is not None else "training")
-        out = RenderFunction.apply(state, norm_planes if kind == ops.DEC_DISENTANGLED else None, planes, scale_src, shift_src, *params)
-        if kind == ops.DEC_OSG:
-            rgb, depth, wsum, _ = out
-            return rgb, None, depth, wsum
-        rgb, seg, depth, wsum, _ = out
-        return rgb, seg, depth, wsum
-
-    @staticmethod
-    def _affine_sources(norm_planes, planes, batch, state):
-        """(scale_src, shift_src) when the differentiable single-gather identity applies to this (norm, planes) pair, else
-        (None, None); sets state['affine_eps'].  The identity replaces the gradient into `planes` by gradients into the
-        normalised planes and the statistics `planes` is tied to (normalize_plane: planes is their root; denormalize_plane:
-        planes is their product), which is only the same thing while the autograd graph still has the shape it had when
-        the pair was made: `planes` must carry grad and `norm_planes` must be in the state it was registered in.  A pair
-        with one branch detached afterwards (renderer(norm.detach(), planes), renderer(norm, planes.detach())) takes the
-        two-gather backward, which honours the detach like the reference does."""
-        if os.environ.get("NFE_BWD_LIBRARY_GEMM", "0") == "1":
-            return None, None
-        src = ops.provenance_sources(norm_planes, planes)
-        if src is None or src[0].numel() != src[2].numel() or src[0].numel() not in (96, 96 * batch):
-            return None, None
-        scale_src, eps, shift_src, norm_rg = src
-        if not planes.requires_grad or bool(norm_planes.requires_grad) != norm_rg:
-            return None, None
-        state["affine_eps"] = eps
-        return scale_src, shift_src
 
     def _render_staged(self, norm_planes, planes, decoder, ray_origins, ray_directions, opts, deterministic):
         """Any decoder callable: the reference's orchestration (renderer.py:99-140,320-363) over the stage
@@ -295,37 +315,25 @@ class ImportanceRenderer(torch.nn.Module):
     def _run_model(self, norm_planes, planes, decoder, sample_coordinates, sample_directions, options):
         desc = self._fused_decoder(decoder, norm_planes)
         if desc is not None:
-            kind, seq_a, seq_b = desc
-            precision = ops.precision_of(options)
             sigma_only = bool(options.get('nfe_sigma_only', False))
             noise = options.get('density_noise', 0) or 0.0
             seed, offset = ops.philox_state(sample_coordinates.device) if noise > 0 else (0, 0)
-            single = (kind == ops.DEC_DISENTANGLED and precision != ops.PRECISIONS['fp32'] and options.get('nfe_single_gather', True)
-                      and self._single_gather_fits(sample_coordinates.shape[1]))
-            if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (norm_planes, planes, *decoder.parameters())):
+            grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (norm_planes, planes, *decoder.parameters()))
+            plan = field_plan("run_model", desc, norm_planes, planes, options, *sample_coordinates.shape[:2], grad, sigma_only)
+            if grad:
                 # differentiable point queries (the density regulariser, loss.py:310-331): autograd.RunModelFunction
                 if sample_coordinates.requires_grad:
                     raise RuntimeError("run_model: gradients w.r.t. sample_coordinates are not built (the reference's callers never ask for them)")
-                from .autograd import RunModelFunction
-                state = {"kind": kind, "seq_a": seq_a, "seq_b": seq_b, "coords": sample_coordinates.detach().float().contiguous(),
-                         "sigma_only": sigma_only,
-                         "cfg": dict(box_warp=options['box_warp'], density_noise=noise, seed=seed, offset=offset, precision=precision)}
-                scale_src, shift_src = self._affine_sources(norm_planes, planes, sample_coordinates.shape[0], state) if single else (None, None)
-                params = [p for seq in (seq_a, seq_b) if seq is not None for p in (seq[0].weight, seq[0].bias, seq[2].weight, seq[2].bias)]
-                outs = RunModelFunction.apply(state, norm_planes if kind == ops.DEC_DISENTANGLED else None, planes, scale_src, shift_src, *params)
-                keys = ("sigma",) if sigma_only else (("rgb", "sigma") if kind == ops.DEC_OSG else ("rgb", "sigma", "seg"))
+                from .autograd import RunModelFunction, _decoder_params
+                args = (sample_coordinates.detach().float().contiguous(), options, seed, offset, sigma_only)
+                outs = RunModelFunction.apply(plan, args, norm_planes if plan.stage_norm else None, planes, *(plan.sources or (None, None)),
+                                              *_decoder_params(plan.seq_a, plan.seq_b))
+                keys = ("sigma",) if sigma_only else (("rgb", "sigma") if plan.kind == ops.DEC_OSG else ("rgb", "sigma", "seg"))
                 return dict(zip(keys, outs))
             ops._no_grad_needed(sample_coordinates)
-            cache = bool(options.get('nfe_cache_planes', False))
-            # density-only queries with the disentangled decoder on the tensor-core path never touch the de-normalised planes
-            geo_only = sigma_only and kind == ops.DEC_DISENTANGLED and precision != ops.PRECISIONS['fp32']
-            affine = ops.provenance(norm_planes, planes) if (single and not geo_only) else None
-            norm_cl = ops.planes_channel_last(norm_planes, cache) if kind == ops.DEC_DISENTANGLED else None
-            denorm_cl = None if (geo_only or affine is not None) else ops.planes_channel_last(planes, cache)
-            ops.note_path("run_model", "single-gather" if (affine is not None or geo_only) else ("two-gather" if kind == ops.DEC_DISENTANGLED else "one-set"))
-            cfg = ops.make_cfg(kind, norm_cl if denorm_cl is None else denorm_cl, 2, 0, options['box_warp'], density_noise=noise, seed=seed,
-                               offset=offset, precision=precision, affine=affine)
-            return ops.run_model_fwd(cfg, seq_a, seq_b, norm_cl, denorm_cl, sample_coordinates, sigma_only=sigma_only)
+            ops.note_path(*plan.path)
+            return run_model_planes(plan, norm_planes, planes, sample_coordinates, options, seed, offset, sigma_only,
+                                    cache=bool(options.get('nfe_cache_planes', False)))[3]
         axes = self.plane_axes
         feats = sample_from_planes(axes, planes, sample_coordinates, padding_mode='zeros', box_warp=options['box_warp'])
         if self._disentangled:

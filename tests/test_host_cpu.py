@@ -246,6 +246,68 @@ def test_plane_registries_are_thread_safe():
     reg.clear()
 
 
+def test_field_plan_decision_table(monkeypatch):
+    """renderer.field_plan over its table: when the single-gather identity applies, geometry-only, which plane sets are
+    staged and which path counter a call records."""
+    from nerffaceediting_b200 import plane_registry as reg
+    from nerffaceediting_b200.renderer import field_plan
+    reg.clear()
+    monkeypatch.delenv("NFE_BWD_LIBRARY_GEMM", raising=False)
+    monkeypatch.delenv("NFE_DEFAULT_PRECISION", raising=False)
+    dis, osg = (ops.DEC_DISENTANGLED, None, None), (ops.DEC_OSG, None, None)
+    norm, raw = torch.randn(2, 96, 4, 4), torch.randn(2, 96, 4, 4)
+    reg.provenance_put(raw, norm, torch.full((2, 96), 2.0), torch.ones(2, 96))
+    n5, r5, other = norm.view(2, 3, 32, 4, 4), raw.view(2, 3, 32, 4, 4), torch.randn(2, 3, 32, 4, 4)
+    opts = dict(depth_resolution=48, depth_resolution_importance=48)
+
+    def plan(what, desc, pair, per_item, grad=False, sigma_only=False, **o):
+        p = field_plan(what, desc, *pair, dict(opts, **o), 2, per_item, grad, sigma_only)
+        return p.affine is not None, p.geo_only, (p.stage_norm, p.stage_denorm), p.path
+
+    single, two = (True, False, (True, False), ("render", "single-gather")), (False, False, (True, True), ("render", "two-gather"))
+    assert plan("render", dis, (n5, r5), 64) == single
+    assert plan("render", dis, (n5, r5), 64, nfe_precision="bf16") == single
+    assert plan("render", dis, (n5, r5), 64, nfe_precision="fp32") == two               # fp32 never uses the identity
+    assert plan("render", dis, (n5, r5), 64, nfe_single_gather=False) == two
+    assert plan("render", dis, (n5, other), 64) == two                                  # no provenance
+    assert plan("render", osg, (None, r5), 64) == (False, False, (False, True), ("render", "one-set"))
+    # 128 samples per item in each pass: rays x min(coarse, fine) for a render, points for run_model
+    assert plan("render", dis, (n5, r5), 3) == single                                   # 3 x 48
+    assert plan("render", dis, (n5, r5), 3, depth_resolution_importance=40) == two      # 3 x 40
+    assert plan("render", dis, (n5, r5), 3, depth_resolution=40) == two                 # 3 x 40
+    assert plan("render", dis, (n5, r5), 2, depth_resolution_importance=0) == two       # 2 x 48, one pass
+    assert plan("render", dis, (n5, r5), 1, depth_resolution=128, depth_resolution_importance=0) == single
+    assert plan("render", dis, (n5, r5), 1, depth_resolution=127, depth_resolution_importance=0) == two
+    assert plan("run_model", dis, (n5, r5), 128)[0] and not plan("run_model", dis, (n5, r5), 127)[0]
+    # geometry-only (sigma-only, disentangled, tensor cores) reads the normalised planes only, with or without provenance
+    geo = (False, True, (True, False), ("run_model", "single-gather"))
+    assert plan("run_model", dis, (n5, r5), 256, sigma_only=True) == geo
+    assert plan("run_model", dis, (n5, other), 256, sigma_only=True) == geo
+    assert plan("run_model", dis, (n5, r5), 256, sigma_only=True, nfe_precision="fp32") == (False, False, (True, True), ("run_model", "two-gather"))
+
+    # training: the identity needs the autograd sources of a registered pair, in the grad state it was registered in
+    raw_t = torch.randn(2, 96, 4, 4, requires_grad=True)
+    mean, std = torch.zeros(2, 96, 1, 1, requires_grad=True), torch.ones(2, 96, 1, 1, requires_grad=True)
+    norm_t = raw_t * 1.0
+    reg.provenance_put(raw_t, norm_t, std.detach().reshape(2, -1) + 1e-8, mean.detach().reshape(2, -1))
+    reg.provenance_attach(raw_t, std, 1e-8, mean)
+    pair = (norm_t.view(2, 3, 32, 4, 4), raw_t.view(2, 3, 32, 4, 4))
+    p = field_plan("render", dis, *pair, opts, 2, 64, True)
+    assert p.sources[0] is std and p.sources[1] is mean and p.path == ("render", "training-single-gather") and not p.stage_denorm
+    assert torch.equal(p.affine[0], std.detach().reshape(2, 96) + 1e-8) and torch.equal(p.affine[1], mean.detach().reshape(2, 96))
+    assert field_plan("run_model", dis, *pair, opts, 2, 256, True).path is None          # training run_model counts nothing
+    refused = (False, False, (True, True), ("render", "training"))
+    assert plan("render", dis, (pair[0].detach(), pair[1]), 64, grad=True) == refused   # norm detached after registration
+    assert plan("render", dis, (pair[0], pair[1].detach()), 64, grad=True) == refused   # planes carry no grad
+    # geometry-only in training still stages the raw planes unless the identity applies: the backward returns their gradient
+    assert plan("run_model", dis, pair, 256, grad=True, sigma_only=True) == (True, True, (True, False), None)
+    assert plan("run_model", dis, (pair[0].detach(), pair[1]), 256, grad=True, sigma_only=True) == (False, True, (True, True), None)
+    monkeypatch.setenv("NFE_BWD_LIBRARY_GEMM", "1")
+    p = field_plan("render", dis, *pair, opts, 2, 64, True)
+    assert p.affine is None and p.sources is None and p.library_gemm and p.path == ("render", "training")
+    reg.clear()
+
+
 def test_missing_library_fails_loudly(monkeypatch):
     monkeypatch.setattr(_lib, "_lib", None)
     monkeypatch.setattr(_lib, "LIB_PATH", "/nonexistent/libnfe_b200.so")
