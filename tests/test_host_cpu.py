@@ -323,6 +323,7 @@ def test_product_never_imports_oracle():
                 src = open(os.path.join(dirpath, f)).read()
                 assert "oracle" not in src.replace("the CPU reference is the oracle", "").replace("(SURVEY.md §7.5, oracle nfo_resample_ray)", "") \
                     .replace("the oracle does not have", ""), f"{f} mentions the oracle"
+                assert "_torch_render" not in src, f"{f} mentions the tests' torch restatement"
 
 
 def test_decoder_recognition_by_structure():
