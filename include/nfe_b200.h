@@ -193,6 +193,11 @@ typedef struct {
     /* nfe_render_fwd only: write rgb / seg as images [n, channel, n_rays] (the feature_image / seg_image
      * of triplane.py:122-125, i.e. after permute(0,2,1).reshape(N,C,H,W)) instead of [n, n_rays, channel]. */
     int image_layout;
+    /* nfe_render_fwd only: geometry without appearance — seg, depth and wsum are computed (bit-identical to the full
+     * render), rgb is neither computed nor written and may be NULL.  The per-sample records shrink to {sigma, seg[15]}
+     * (16 floats; none for NFE_DEC_OSG, whose field pass writes sigma alone); with the disentangled decoder app_net and
+     * the de-normalised planes are not touched (planes_denorm_cl may be NULL, affine_* are ignored). */
+    int geometry_only;
 } nfe_render_cfg;
 
 /* bytes of device workspace nfe_render_fwd needs for n*n_rays rays with this cfg */
@@ -215,7 +220,7 @@ int nfe_render_fwd(const nfe_render_cfg* cfg, const nfe_mlp* net_a, const nfe_ml
 
 /* Byte offsets, inside an nfe_render_fwd workspace, of what the backward pass re-reads:
  * offsets[0..3] = sigma_c [T,s_c], rec_c [T,s_c,48], sigma_f [T,s_f], rec_f [T,s_f,48] (-1 if absent);
- * a record is {sigma, seg[15], rgb[32]}. */
+ * a record is {sigma, seg[15], rgb[32]}.  A geometry_only cfg is rejected: no backward reads its workspace. */
 int nfe_render_workspace_layout(const nfe_render_cfg* cfg, int n, int64_t n_rays, int64_t* offsets);
 
 /* ---- backward (BASELINE config 4).  Gradients flow to the plane tensors and the decoder parameters only;

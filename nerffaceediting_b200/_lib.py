@@ -32,7 +32,8 @@ class NfeRenderCfg(ctypes.Structure):
                 ("s_c", c_int), ("s_f", c_int), ("color_dim", c_int), ("seg_dim", c_int),
                 ("white_back", c_int), ("box_warp", c_float), ("density_noise", c_float),
                 ("stochastic", c_int), ("seed", c_u64), ("offset", c_u64), ("precision", c_int),
-                ("affine_scale", c_vp), ("affine_shift", c_vp), ("affine_items", c_int), ("sigma_only", c_int), ("image_layout", c_int)]
+                ("affine_scale", c_vp), ("affine_shift", c_vp), ("affine_items", c_int), ("sigma_only", c_int), ("image_layout", c_int),
+                ("geometry_only", c_int)]
 
 
 class NfeModconvArgs(ctypes.Structure):

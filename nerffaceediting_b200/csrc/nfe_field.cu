@@ -104,17 +104,21 @@ __global__ void __launch_bounds__(256, 1) decoder_kernel(nfe_mlp net_a, nfe_mlp 
 //            swizzled shared tile;
 //   phase 2  one sample per lane: both MLPs from registers, parameters broadcast from shared;
 //   phase 3  results staged through the same tile and written out coalesced.
+// GEO: the geometry-only render pass (FieldArgs::geometry_only) — 16-float records {sigma, seg[15]}, no colours; with the
+// disentangled decoder only the normalised planes are gathered and app_net is not run.  Its own instantiation, so the
+// full kernels keep their code.
 // ------------------------------------------------------------------------------------------
-template <int KIND>
+template <int KIND, bool GEO>
 __global__ void __launch_bounds__(FIELD_THREADS, 1) field_kernel(FieldArgs a, nfe_mlp net_a, nfe_mlp net_b)
 {
     using T = DecoderTraits<KIND>;
+    constexpr bool NORM_ONLY = GEO && KIND == NFE_DEC_DISENTANGLED;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     MlpParams<T::OUT_A>& pa = *reinterpret_cast<MlpParams<T::OUT_A>*>(smem_raw);
     MlpParams<T::OUT_B>& pb = *reinterpret_cast<MlpParams<T::OUT_B>*>(smem_raw + sizeof(MlpParams<T::OUT_A>));
     float4* tiles = reinterpret_cast<float4*>(smem_raw + sizeof(MlpParams<T::OUT_A>) + sizeof(MlpParams<T::OUT_B>));
     load_mlp(pa, net_a);
-    if (T::HAS_B) load_mlp(pb, net_b);
+    if (T::HAS_B && !NORM_ONLY) load_mlp(pb, net_b);
     __syncthreads();
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -149,12 +153,12 @@ __global__ void __launch_bounds__(FIELD_THREADS, 1) field_kernel(FieldArgs a, nf
                 const TapSet ts = make_tapset(taps3(__fmul_rn(a.scale, x), __fmul_rn(a.scale, y), __fmul_rn(a.scale, z), a.H, a.W), a.H, a.W);
                 float4 va[12], vb[12];
                 if (T::SETS == 2) gather_load(a.set_norm + pbi * set_stride, ts, c4, va);
-                gather_load(a.set_denorm + pbi * set_stride, ts, c4, vb);
+                if (!NORM_ONLY) gather_load(a.set_denorm + pbi * set_stride, ts, c4, vb);
                 if (T::SETS == 2) fa = gather_reduce(va, ts);
-                fb = gather_reduce(vb, ts);
+                if (!NORM_ONLY) fb = gather_reduce(vb, ts);
             }
             if (T::SETS == 2) tile[tile_chunk(row, c4)] = fa;
-            tile[256 + tile_chunk(row, c4)] = fb;
+            if (!NORM_ONLY) tile[256 + tile_chunk(row, c4)] = fb;
         }
         __syncwarp();
 
@@ -174,12 +178,12 @@ __global__ void __launch_bounds__(FIELD_THREADS, 1) field_kernel(FieldArgs a, nf
             if constexpr (KIND == NFE_DEC_DISENTANGLED) {
 #pragma unroll
                 for (int c = 0; c < 15; ++c) segv[c] = outa[1 + c];
-            } else {
+            } else if constexpr (!GEO) {
 #pragma unroll
                 for (int c = 0; c < 32; ++c) col[c] = rgb_activation(outa[1 + c]);
             }
         }
-        if constexpr (T::HAS_B) {
+        if constexpr (T::HAS_B && !NORM_ONLY) {
             if constexpr (T::SETS == 2) {
 #pragma unroll
                 for (int c = 0; c < 8; ++c) {
@@ -210,12 +214,17 @@ __global__ void __launch_bounds__(FIELD_THREADS, 1) field_kernel(FieldArgs a, nf
 #pragma unroll
             for (int c = 0; c < 15; ++c) row[1 + c] = segv[c];
         }
+        if constexpr (!GEO) {
 #pragma unroll
-        for (int c = 0; c < 32; ++c) row[17 + c] = col[c];
+            for (int c = 0; c < 32; ++c) row[17 + c] = col[c];
+        }
         __syncwarp();
         const int rows = (int)min((int64_t)32, a.total - base);
         if (lane < rows) a.sigma[base + lane] = row[0];
-        if (a.sigma_only) {
+        if constexpr (GEO) {
+            // geometry records {sigma, seg[15]}: 16 floats per sample, the whole step is one contiguous span
+            for (int e = lane; e < rows * 16; e += 32) a.rec[base * 16 + e] = tile_f[(e >> 4) * OUT_STRIDE + (e & 15)];
+        } else if (a.sigma_only) {
             // density-only query: nothing else is written
         } else if (a.rec) {
             // packed records {sigma, seg[15], rgb[32]}: 48 floats per sample, the whole step is one contiguous span
@@ -233,21 +242,21 @@ __global__ void __launch_bounds__(FIELD_THREADS, 1) field_kernel(FieldArgs a, nf
     }
 }
 
-template <int KIND>
+template <int KIND, bool GEO>
 static int launch_field_kind(const FieldArgs& a, const nfe_mlp& net_a, const nfe_mlp& net_b, cudaStream_t stream)
 {
     using T = DecoderTraits<KIND>;
     const size_t smem = sizeof(MlpParams<T::OUT_A>) + sizeof(MlpParams<T::OUT_B>) + (size_t)(FIELD_THREADS / 32) * 8192;
     static bool configured = false;
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(field_kernel<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(field_kernel<KIND, GEO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) { set_error("field_kernel: cannot reserve %zu bytes of shared memory: %s", smem, cudaGetErrorString(e)); return 2; }
         configured = true;
     }
     const int64_t n_steps = (a.total + 31) / 32;
     const int64_t blocks_needed = (n_steps + FIELD_THREADS / 32 - 1) / (FIELD_THREADS / 32);
     const unsigned grid = (unsigned)(blocks_needed < sm_count() ? blocks_needed : sm_count());
-    field_kernel<KIND><<<grid, FIELD_THREADS, smem, stream>>>(a, net_a, net_b);
+    field_kernel<KIND, GEO><<<grid, FIELD_THREADS, smem, stream>>>(a, net_a, net_b);
     return check_launch("field_kernel");
 }
 
@@ -268,7 +277,7 @@ int check_decoder_dims(int kind, const nfe_mlp* net_a, const nfe_mlp* net_b, con
 }
 
 int field_planes(const nfe_render_cfg* cfg, const float* planes_norm_cl, const float* planes_denorm_cl, int plane_batch, int n,
-                 int64_t pass_samples, bool sigma_only, const char* who, FieldArgs& f)
+                 int64_t pass_samples, bool sigma_only, bool geometry_only, const char* who, FieldArgs& f)
 {
     NFE_REQUIRE(cfg->channels == FEAT, "%s: planes must have %d channels (got %d)", who, FEAT, cfg->channels);
     NFE_REQUIRE(cfg->height >= 1 && cfg->width >= 1, "%s: bad plane size", who);
@@ -276,10 +285,12 @@ int field_planes(const nfe_render_cfg* cfg, const float* planes_norm_cl, const f
     NFE_REQUIRE(cfg->precision >= NFE_PREC_FP32 && cfg->precision <= NFE_PREC_BF16, "%s: unknown precision mode %d", who, cfg->precision);
     NFE_REQUIRE(cfg->seg_dim == (cfg->kind == NFE_DEC_OSG ? 0 : 15), "%s: seg_dim %d unsupported for decoder kind %d", who, cfg->seg_dim, cfg->kind);
     const bool disentangled_tc = cfg->kind == NFE_DEC_DISENTANGLED && cfg->precision != NFE_PREC_FP32;
+    // a geometry-only render with the disentangled decoder needs geo_net on the normalised planes alone (every precision)
+    const bool norm_only = geometry_only && cfg->kind == NFE_DEC_DISENTANGLED;
     // single-gather identity (cfg->affine_*): the de-normalised planes are norm*scale + shift and are not read
-    const bool affine = cfg->affine_scale && cfg->affine_shift && disentangled_tc;
+    const bool affine = cfg->affine_scale && cfg->affine_shift && disentangled_tc && !norm_only;
     // a density-only query with the disentangled decoder on the tensor cores reads the normalised planes only
-    const bool geo_only = sigma_only && disentangled_tc;
+    const bool geo_only = (sigma_only && disentangled_tc) || norm_only;
     NFE_REQUIRE(!cfg->affine_scale || cfg->affine_items == 1 || cfg->affine_items == n, "%s: affine statistics for %d items, batch is %d", who,
                 cfg->affine_items, n);
     // the field kernel keeps the statistics of two batch items per 128-sample tile: an item must span at least one tile in each pass
@@ -291,7 +302,9 @@ int field_planes(const nfe_render_cfg* cfg, const float* planes_norm_cl, const f
     f.set_norm = planes_norm_cl; f.set_denorm = planes_denorm_cl; f.plane_batch = plane_batch; f.H = cfg->height; f.W = cfg->width;
     f.scale = (float)(2.0 / (double)cfg->box_warp);
     if (affine) { f.affine_scale = cfg->affine_scale; f.affine_shift = cfg->affine_shift; f.affine_items = cfg->affine_items; }
-    f.sigma_only = sigma_only;
+    // the OSG decoder has no semantics: its geometry-only pass is a density-only one (no records)
+    f.sigma_only = sigma_only || (geometry_only && cfg->kind == NFE_DEC_OSG);
+    f.geometry_only = geometry_only && cfg->kind != NFE_DEC_OSG;
     return 0;
 }
 
@@ -303,10 +316,15 @@ int launch_field(int kind, int precision, const FieldArgs& a, const nfe_mlp* net
                 a.plane_batch, a.H, a.W);
     if (precision != NFE_PREC_FP32) return launch_field_pipe2(kind, precision, a, net_a, net_b, stream);
     nfe_mlp none = {};
+    if (a.geometry_only) {
+        NFE_REQUIRE(kind != NFE_DEC_OSG && a.rec, "field kernel: a geometry-only pass needs a decoder with semantics and the records");
+        if (kind == NFE_DEC_DISENTANGLED) return launch_field_kind<NFE_DEC_DISENTANGLED, true>(a, *net_a, *net_b, stream);
+        return launch_field_kind<NFE_DEC_SEGMENTATION, true>(a, *net_a, *net_b, stream);
+    }
     switch (kind) {
-        case NFE_DEC_OSG: return launch_field_kind<NFE_DEC_OSG>(a, *net_a, none, stream);
-        case NFE_DEC_DISENTANGLED: return launch_field_kind<NFE_DEC_DISENTANGLED>(a, *net_a, *net_b, stream);
-        default: return launch_field_kind<NFE_DEC_SEGMENTATION>(a, *net_a, *net_b, stream);
+        case NFE_DEC_OSG: return launch_field_kind<NFE_DEC_OSG, false>(a, *net_a, none, stream);
+        case NFE_DEC_DISENTANGLED: return launch_field_kind<NFE_DEC_DISENTANGLED, false>(a, *net_a, *net_b, stream);
+        default: return launch_field_kind<NFE_DEC_SEGMENTATION, false>(a, *net_a, *net_b, stream);
     }
 }
 
@@ -382,7 +400,7 @@ NFE_EXPORT int nfe_run_model_fwd(const nfe_render_cfg* cfg, const nfe_mlp* net_a
     if ((int64_t)n * m == 0) return 0;
     const bool sigma_only = cfg->sigma_only != 0;
     FieldArgs a = {};
-    if (int rc = field_planes(cfg, planes_norm_cl, planes_denorm_cl, plane_batch, n, m, sigma_only, "nfe_run_model_fwd", a)) return rc;
+    if (int rc = field_planes(cfg, planes_norm_cl, planes_denorm_cl, plane_batch, n, m, sigma_only, false, "nfe_run_model_fwd", a)) return rc;
     NFE_REQUIRE(coords && sigma && (rgb || sigma_only), "nfe_run_model_fwd: null pointer");
     NFE_REQUIRE(cfg->kind == NFE_DEC_OSG || seg || sigma_only, "nfe_run_model_fwd: seg output missing");
     a.coords = coords; a.m = m; a.total = (int64_t)n * m; a.s_per_ray = 1;

@@ -33,14 +33,19 @@ struct FieldArgs {
     float density_noise;
     uint64_t seed, offset;
     int sigma_only;           // write sigma only (rgb / seg / rec untouched); the pipelined kernel also skips the work behind them
+    // Geometry-only render pass (segmentation / disentangled decoders): rec rows are {sigma, seg[15]} (16 floats, 64 bytes)
+    // and no colour is computed; the disentangled decoder reads set_norm alone.  (Sits in the struct's tail padding: the
+    // kernels' parameter layout is unchanged.)
+    int geometry_only;
 };
 
 int check_decoder_dims(int kind, const nfe_mlp* net_a, const nfe_mlp* net_b, const char* who);
 // Checks the cfg fields that nfe_render_fwd and nfe_run_model_fwd share and fills the plane half of `f`: plane sets, plane batch,
 // size, 2/box_warp and, under the single-gather identity, the statistics.  pass_samples: samples per batch item in the smaller
-// pass; sigma_only: a density-only query.  Error messages start with `who`.
+// pass; sigma_only: a density-only query; geometry_only: a geometry-only render pass (sigma alone for the OSG decoder).
+// Error messages start with `who`.
 int field_planes(const nfe_render_cfg* cfg, const float* planes_norm_cl, const float* planes_denorm_cl, int plane_batch, int n,
-                 int64_t pass_samples, bool sigma_only, const char* who, FieldArgs& f);
+                 int64_t pass_samples, bool sigma_only, bool geometry_only, const char* who, FieldArgs& f);
 // precision: NFE_PREC_FP32 -> SIMT fp32 kernel (nfe_field.cu); NFE_PREC_BF16X3 / NFE_PREC_BF16 -> the tcgen05 kernel
 // (nfe_field_pipe2.cu)
 int launch_field(int kind, int precision, const FieldArgs& a, const nfe_mlp* net_a, const nfe_mlp* net_b, cudaStream_t stream);

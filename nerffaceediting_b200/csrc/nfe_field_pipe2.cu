@@ -237,7 +237,10 @@ __device__ __forceinline__ void regs_inc() { asm volatile("setmaxnreg.inc.sync.a
 template <int REGS>
 __device__ __forceinline__ void regs_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" :: "n"(REGS)); }
 
-template <int KIND, bool SPLIT>
+// GEO: the geometry-only render pass (FieldArgs::geometry_only): 16-float records {sigma, seg[15]} and no colour work — the
+// disentangled decoder runs geo_net on the normalised planes alone (the skip_b path of sigma_only, logits kept), the
+// segmentation decoder keeps net's sigma column and seg_net.  A separate instantiation: the full kernels keep their code.
+template <int KIND, bool SPLIT, bool GEO>
 __global__ void __launch_bounds__(THREADS, 1) field_pipe2_kernel(FieldArgs a, nfe_mlp net_a, nfe_mlp net_b)
 {
     using T = TcTraits<KIND>;
@@ -280,7 +283,7 @@ __global__ void __launch_bounds__(THREADS, 1) field_pipe2_kernel(FieldArgs a, nf
     const int n_my = (int)((n_tiles - blockIdx.x + G - 1) / G);
     // sigma_only with the disentangled decoder: sigma is output 0 of geo_net on the normalised planes, so the
     // de-normalised gather and the whole appearance net are skipped
-    const bool skip_b = a.sigma_only && KIND == NFE_DEC_DISENTANGLED;
+    const bool skip_b = (GEO || a.sigma_only) && KIND == NFE_DEC_DISENTANGLED;
     const bool has_b = T::HAS_B && !skip_b;
 #ifdef NFE_PIPE_PROFILE
     long long prof_[16] = {};
@@ -529,7 +532,9 @@ __global__ void __launch_bounds__(THREADS, 1) field_pipe2_kernel(FieldArgs a, nf
         {
             const bool leader = tc::elect_one();
             constexpr uint32_t idesc1 = tc::make_idesc_bf16(TILE_M, HIDDEN);
-            constexpr uint32_t idesc2a = tc::make_idesc_bf16(TILE_M, T::N_A);
+            // geometry: net A's layer 2 only for its first 16 columns (sigma and, for the disentangled decoder, the logits; the
+            // segmentation decoder's 32 colour columns are not computed)
+            constexpr uint32_t idesc2a = tc::make_idesc_bf16(TILE_M, GEO ? 16 : T::N_A);
             constexpr uint32_t idesc2b = tc::make_idesc_bf16(TILE_M, T::N_B);
             // layer 1 of tile `it` into the accumulator set of its group (= ring slot = it & 1)
             auto layer1 = [&](int it) {
@@ -627,7 +632,7 @@ __global__ void __launch_bounds__(THREADS, 1) field_pipe2_kernel(FieldArgs a, nf
                     }
                 }
                 done = a.sigma_only;
-                if (!done) {
+                if (!done && !GEO) {
                     P2_WAIT(10, &s.d2b_full[gi], ph);
                     tc::fence_after_sync();
 #pragma unroll 1
@@ -648,7 +653,7 @@ __global__ void __launch_bounds__(THREADS, 1) field_pipe2_kernel(FieldArgs a, nf
                 // OSG / segmentation decoders (sigma shares net A's output row with the colours): straight-line code
                 float outa[T::N_A];
 #pragma unroll
-                for (int q = 0; q < T::N_A / 16; ++q) {
+                for (int q = 0; q < (GEO ? 1 : T::N_A / 16); ++q) {       // geometry: sigma is in the first 16 columns
                     float v[16];
                     tc::tmem_ld16(lane_addr + COL_D2 + q * 16, v);
                     tc::tmem_ld_wait();
@@ -670,10 +675,12 @@ __global__ void __launch_bounds__(THREADS, 1) field_pipe2_kernel(FieldArgs a, nf
                         rec[0] = make_float4(sig, 0.f, 0.f, 0.f);
                         rec[1] = rec[2] = rec[3] = make_float4(0.f, 0.f, 0.f, 0.f);
                     }
+                    if constexpr (!GEO) {
 #pragma unroll
-                    for (int c = 0; c < 8; ++c)
-                        rec[4 + c] = make_float4(rgb_activation(outa[1 + 4 * c]), rgb_activation(outa[2 + 4 * c]),
-                                                 rgb_activation(outa[3 + 4 * c]), rgb_activation(outa[4 + 4 * c]));
+                        for (int c = 0; c < 8; ++c)
+                            rec[4 + c] = make_float4(rgb_activation(outa[1 + 4 * c]), rgb_activation(outa[2 + 4 * c]),
+                                                     rgb_activation(outa[3 + 4 * c]), rgb_activation(outa[4 + 4 * c]));
+                    }
                     if constexpr (T::HAS_B) {
                         P2_WAIT(10, &s.d2b_full[gi], ph);
                         tc::fence_after_sync();
@@ -703,7 +710,15 @@ __global__ void __launch_bounds__(THREADS, 1) field_pipe2_kernel(FieldArgs a, nf
                 const int64_t L0 = tile * TILE_M + wq * 32;
                 const int n_rows = (int)min((int64_t)32, a.total - L0);
                 const unsigned char* rows = s.recbuf[gi][wq * 32];
-                if (a.rec) {
+                if constexpr (GEO) {
+                    float4* gdst = reinterpret_cast<float4*>(a.rec + L0 * 16);
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) {                      // chunk k*32 + lane = row 8k + lane/4, 16-byte chunk lane%4
+                        const int r = 8 * k + (lane >> 2);
+                        const float4 v = *reinterpret_cast<const float4*>(rows + r * REC_STAGE_STRIDE + (lane & 3) * 16);
+                        if (r < n_rows) gdst[k * 32 + lane] = v;
+                    }
+                } else if (a.rec) {
                     float4* gdst = reinterpret_cast<float4*>(a.rec + L0 * 48);
                     int r = lane / 12, c = lane % 12;                  // chunk k*32 + lane = row r, 16-byte chunk c of the record
 #pragma unroll 4
@@ -752,19 +767,19 @@ __global__ void __launch_bounds__(THREADS, 1) field_pipe2_kernel(FieldArgs a, nf
     if (warp == MMA_WARP) tc::tmem_dealloc(tmem, P2_TMEM_COLS);
 }
 
-template <int KIND, bool SPLIT>
+template <int KIND, bool SPLIT, bool GEO>
 static int launch_kind(const FieldArgs& a, const nfe_mlp& net_a, const nfe_mlp& net_b, cudaStream_t stream)
 {
     const size_t smem = sizeof(Smem<KIND, SPLIT>) + 128;
     static bool configured = false;
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(field_pipe2_kernel<KIND, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(field_pipe2_kernel<KIND, SPLIT, GEO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) { set_error("field_pipe2_kernel: cannot reserve %zu bytes of shared memory: %s", smem, cudaGetErrorString(e)); return 2; }
         configured = true;
     }
     const int64_t n_tiles = (a.total + TILE_M - 1) / TILE_M;
     const int64_t cap = sm_count();   // persistent: one CTA per SM (it owns all 512 TMEM columns)
-    field_pipe2_kernel<KIND, SPLIT><<<(unsigned)(n_tiles < cap ? n_tiles : cap), THREADS, smem, stream>>>(a, net_a, net_b);
+    field_pipe2_kernel<KIND, SPLIT, GEO><<<(unsigned)(n_tiles < cap ? n_tiles : cap), THREADS, smem, stream>>>(a, net_a, net_b);
     return check_launch("field_pipe2_kernel");
 }
 
@@ -775,15 +790,24 @@ int launch_field_pipe2(int kind, int precision, const FieldArgs& a, const nfe_ml
     if (a.total <= 0) return 0;
     nfe_mlp none = {};
     const bool split = precision == NFE_PREC_BF16X3;
+    if (a.geometry_only) {
+        NFE_REQUIRE(kind != NFE_DEC_OSG && a.rec, "field_pipe2_kernel: a geometry-only pass needs a decoder with semantics and the records");
+        if (kind == NFE_DEC_DISENTANGLED)
+            return split ? p2::launch_kind<NFE_DEC_DISENTANGLED, true, true>(a, *net_a, *net_b, stream)
+                         : p2::launch_kind<NFE_DEC_DISENTANGLED, false, true>(a, *net_a, *net_b, stream);
+        return split ? p2::launch_kind<NFE_DEC_SEGMENTATION, true, true>(a, *net_a, *net_b, stream)
+                     : p2::launch_kind<NFE_DEC_SEGMENTATION, false, true>(a, *net_a, *net_b, stream);
+    }
     switch (kind) {
         case NFE_DEC_OSG:
-            return split ? p2::launch_kind<NFE_DEC_OSG, true>(a, *net_a, none, stream) : p2::launch_kind<NFE_DEC_OSG, false>(a, *net_a, none, stream);
+            return split ? p2::launch_kind<NFE_DEC_OSG, true, false>(a, *net_a, none, stream)
+                         : p2::launch_kind<NFE_DEC_OSG, false, false>(a, *net_a, none, stream);
         case NFE_DEC_DISENTANGLED:
-            return split ? p2::launch_kind<NFE_DEC_DISENTANGLED, true>(a, *net_a, *net_b, stream)
-                         : p2::launch_kind<NFE_DEC_DISENTANGLED, false>(a, *net_a, *net_b, stream);
+            return split ? p2::launch_kind<NFE_DEC_DISENTANGLED, true, false>(a, *net_a, *net_b, stream)
+                         : p2::launch_kind<NFE_DEC_DISENTANGLED, false, false>(a, *net_a, *net_b, stream);
         default:
-            return split ? p2::launch_kind<NFE_DEC_SEGMENTATION, true>(a, *net_a, *net_b, stream)
-                         : p2::launch_kind<NFE_DEC_SEGMENTATION, false>(a, *net_a, *net_b, stream);
+            return split ? p2::launch_kind<NFE_DEC_SEGMENTATION, true, false>(a, *net_a, *net_b, stream)
+                         : p2::launch_kind<NFE_DEC_SEGMENTATION, false, false>(a, *net_a, *net_b, stream);
     }
 }
 

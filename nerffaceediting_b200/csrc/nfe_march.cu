@@ -76,9 +76,18 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 // c3 1.89 -> 1.72 ms, c5 28.7 -> 25.9 ms; 4 / 12 / 16 groups: 0.135 / 0.130 / 0.143).
 constexpr int MARCH_RING_GROUPS = 4;    // groups (of 2*MARCH_GROUP_PAIRS rows) in a warp's record ring: 16 rows = 3 KB per warp (6 groups: no better)
 constexpr int MARCH_MIN_BLOCKS = 4;     // 64 registers: 4 blocks per SM keep more record rows in flight (merge+composite at c2: 0.157 -> 0.142 ms; 5 is slower)
-template <bool SORT>
+// Geometry records {sigma, seg[15]} (GEO, a geometry-only render: rec1 with cc == 0) are 64-byte rows; their ring keeps the same
+// 3 KB per warp in flight (48 rows).
+constexpr int MARCH_RING_GROUPS_GEO = 12;
+// record row: 12 float4 {sigma, seg[15], rgb[32]}, or 4 float4 {sigma, seg[15]} (GEO); ring groups and their bytes
+template <bool GEO> struct MarchRing {
+    static constexpr int ROW_F4 = GEO ? 4 : 12, ROW_BYTES = ROW_F4 * 16;
+    static constexpr int GROUPS = GEO ? MARCH_RING_GROUPS_GEO : MARCH_RING_GROUPS, GROUP_BYTES = MARCH_GROUP_PAIRS * 2 * ROW_BYTES;
+};
+template <bool SORT, bool GEO>
 __global__ void __launch_bounds__(256, MARCH_MIN_BLOCKS) march_kernel(MarchArgs a)
 {
+    using R = MarchRing<GEO>;
     extern __shared__ __align__(16) float smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int warps_per_block = blockDim.x >> 5;
@@ -100,21 +109,21 @@ __global__ void __launch_bounds__(256, MARCH_MIN_BLOCKS) march_kernel(MarchArgs 
         //      sum_e omega'_e c_e with omega' scattered by entry), so their addresses are known before the merge: the first
         //      MARCH_RING_GROUPS groups are requested here with cp.async and land while the merge and the scans run
         const int rg_half = lane >> 4, rg_q = lane & 15;
-        const bool rg_on = rg_q < 12;
+        const bool rg_on = rg_q < R::ROW_F4;
         const float4* rg_r1 = nullptr;
         const float4* rg_r2 = nullptr;
         uint32_t rg_slot0 = 0;
         if (a.rec1) {
-            rg_r1 = reinterpret_cast<const float4*>(a.rec1 + ray * a.s1 * 48) + rg_q;
-            rg_r2 = a.s2 ? reinterpret_cast<const float4*>(a.rec2 + (ray * a.s2 - a.s1) * 48) + rg_q : rg_r1;
+            rg_r1 = reinterpret_cast<const float4*>(a.rec1 + ray * a.s1 * (4 * R::ROW_F4)) + rg_q;
+            rg_r2 = a.s2 ? reinterpret_cast<const float4*>(a.rec2 + (ray * a.s2 - a.s1) * (4 * R::ROW_F4)) + rg_q : rg_r1;
             char* ring_base = reinterpret_cast<char*>(smem) + (((size_t)warps_per_block * MARCH_SMEM_FLOATS_PER_SAMPLE * S * 4 + 15) & ~(size_t)15)
-                              + (size_t)warp * MARCH_RING_GROUPS * MARCH_RING_GROUP_BYTES;
-            rg_slot0 = (uint32_t)__cvta_generic_to_shared(ring_base) + (uint32_t)(rg_half * 192 + rg_q * 16);
-            for (int g = 0; g < MARCH_RING_GROUPS; ++g) {
+                              + (size_t)warp * R::GROUPS * R::GROUP_BYTES;
+            rg_slot0 = (uint32_t)__cvta_generic_to_shared(ring_base) + (uint32_t)(rg_half * R::ROW_BYTES + rg_q * 16);
+            for (int g = 0; g < R::GROUPS; ++g) {
 #pragma unroll
                 for (int j = 0; j < MARCH_GROUP_PAIRS; ++j) {
                     const int e = 2 * (MARCH_GROUP_PAIRS * g + j) + rg_half;
-                    if (rg_on && e < S) cp_async16(rg_slot0 + g * MARCH_RING_GROUP_BYTES + j * 384, (e < a.s1 ? rg_r1 : rg_r2) + e * 12);
+                    if (rg_on && e < S) cp_async16(rg_slot0 + g * R::GROUP_BYTES + j * 2 * R::ROW_BYTES, (e < a.s1 ? rg_r1 : rg_r2) + e * R::ROW_F4);
                 }
                 cp_async_commit();
             }
@@ -185,11 +194,12 @@ __global__ void __launch_bounds__(256, MARCH_MIN_BLOCKS) march_kernel(MarchArgs 
         // ---- channel sums
         if (a.rec1) {
             // Packed records (48 floats = 12 float4 per sample): a half-warp reads one whole 192-byte row per load,
-            // lanes 0-11 take the even rows, lanes 16-27 the odd ones; the two halves are added at the end.
+            // lanes 0-11 take the even rows, lanes 16-27 the odd ones; the two halves are added at the end.  Geometry records
+            // (16 floats) go the same way with lanes 0-3 / 16-19, so seg sums in exactly the full render's order.
             for (int k = lane; k < S; k += 32) s_sigma[k] = 0.5f * ((k > 0 ? s_w[k - 1] : 0.0f) + (k < n_int ? s_w[k] : 0.0f));
             __syncwarp();
             const int half = lane >> 4, q = lane & 15;
-            const bool on = q < 12;
+            const bool on = q < R::ROW_F4;
             float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
             // omega by entry (s_raw is free after the merge), then walk the ring: group g holds 2*MARCH_GROUP_PAIRS consecutive rows in memory order;
             // every lane reads back exactly the 16 bytes it requested itself, so cp.async.wait_group is all the ordering needed
@@ -198,30 +208,30 @@ __global__ void __launch_bounds__(256, MARCH_MIN_BLOCKS) march_kernel(MarchArgs 
             const int n_groups = (S + 2 * MARCH_GROUP_PAIRS - 1) / (2 * MARCH_GROUP_PAIRS);
             int slot = 0;
             for (int g = 0; g < n_groups; ++g) {
-                cp_async_wait<MARCH_RING_GROUPS - 1>();       // MARCH_RING_GROUPS groups were committed after group g-1: g has landed
+                cp_async_wait<R::GROUPS - 1>();             // R::GROUPS groups were committed after group g-1: g has landed
 #pragma unroll
                 for (int j = 0; j < MARCH_GROUP_PAIRS; ++j) {
                     const int e = 2 * (MARCH_GROUP_PAIRS * g + j) + rg_half;
                     if (rg_on && e < S) {
                         float4 v;
                         asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w)
-                                     : "r"(rg_slot0 + slot * MARCH_RING_GROUP_BYTES + j * 384) : "memory");
+                                     : "r"(rg_slot0 + slot * R::GROUP_BYTES + j * 2 * R::ROW_BYTES) : "memory");
                         const float om = s_raw[e];
                         acc.x = fmaf(om, v.x, acc.x); acc.y = fmaf(om, v.y, acc.y); acc.z = fmaf(om, v.z, acc.z); acc.w = fmaf(om, v.w, acc.w);
                     }
                 }
 #pragma unroll
                 for (int j = 0; j < MARCH_GROUP_PAIRS; ++j) {   // refill the slot just consumed
-                    const int e2 = 2 * (MARCH_GROUP_PAIRS * (g + MARCH_RING_GROUPS) + j) + rg_half;
-                    if (rg_on && e2 < S) cp_async16(rg_slot0 + slot * MARCH_RING_GROUP_BYTES + j * 384, (e2 < a.s1 ? rg_r1 : rg_r2) + e2 * 12);
+                    const int e2 = 2 * (MARCH_GROUP_PAIRS * (g + R::GROUPS) + j) + rg_half;
+                    if (rg_on && e2 < S) cp_async16(rg_slot0 + slot * R::GROUP_BYTES + j * 2 * R::ROW_BYTES, (e2 < a.s1 ? rg_r1 : rg_r2) + e2 * R::ROW_F4);
                 }
                 cp_async_commit();
-                slot = slot + 1 == MARCH_RING_GROUPS ? 0 : slot + 1;
+                slot = slot + 1 == R::GROUPS ? 0 : slot + 1;
             }
             acc.x += __shfl_xor_sync(0xffffffffu, acc.x, 16); acc.y += __shfl_xor_sync(0xffffffffu, acc.y, 16);
             acc.z += __shfl_xor_sync(0xffffffffu, acc.z, 16); acc.w += __shfl_xor_sync(0xffffffffu, acc.w, 16);
             if (half == 0 && on) {
-                if (q >= 4) {                                   // rgb channels 4(q-4) .. +3
+                if (!GEO && q >= 4) {                           // rgb channels 4(q-4) .. +3
                     if (a.white_back) { const float bg = 1.0f - wt; acc.x += bg; acc.y += bg; acc.z += bg; acc.w += bg; }
                     const float4 o4 = make_float4(acc.x * 2.0f - 1.0f, acc.y * 2.0f - 1.0f, acc.z * 2.0f - 1.0f, acc.w * 2.0f - 1.0f);
                     if (a.image_rays) {
@@ -506,17 +516,26 @@ int launch_march(const MarchArgs& a, bool sort, cudaStream_t stream)
     if (a.n_rays <= 0) return 0;
     const int warps = warps_for(S, MARCH_SMEM_FLOATS_PER_SAMPLE);
     size_t smem = (size_t)warps * MARCH_SMEM_FLOATS_PER_SAMPLE * 4 * S;
-    // packed records: cp.async ring of MARCH_RING_GROUPS groups per warp behind the scan arrays
-    if (a.rec1) smem = ((smem + 15) & ~(size_t)15) + (size_t)warps * MARCH_RING_GROUPS * MARCH_RING_GROUP_BYTES;
+    // packed records: cp.async ring behind the scan arrays; records without colours are the geometry-only render's
+    const bool geo = a.rec1 && a.cc == 0;
+    NFE_REQUIRE(!a.rec1 || a.cc == 32 || (geo && a.cs == 15), "ray march: packed records carry 32 colours, or 15 semantic channels alone");
+    if (a.rec1)
+        smem = ((smem + 15) & ~(size_t)15) + (size_t)warps * (geo ? MarchRing<true>::GROUPS * MarchRing<true>::GROUP_BYTES
+                                                                  : MarchRing<false>::GROUPS * MarchRing<false>::GROUP_BYTES);
     const int64_t blocks = (a.n_rays + warps - 1) / warps;
     const int64_t cap = (int64_t)sm_count() * 8;
     const unsigned grid = (unsigned)(blocks < cap ? blocks : cap);
-    if (sort) {
-        if (smem > SMEM_OPT_IN) cudaFuncSetAttribute(march_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        march_kernel<true><<<grid, warps * 32, smem, stream>>>(a);
+    auto launch = [&](auto kernel) {
+        if (smem > SMEM_OPT_IN) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        kernel<<<grid, warps * 32, smem, stream>>>(a);
+    };
+    if (geo) {
+        if (sort) launch(march_kernel<true, true>);
+        else launch(march_kernel<false, true>);
+    } else if (sort) {
+        launch(march_kernel<true, false>);
     } else {
-        if (smem > SMEM_OPT_IN) cudaFuncSetAttribute(march_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        march_kernel<false><<<grid, warps * 32, smem, stream>>>(a);
+        launch(march_kernel<false, false>);
     }
     return check_launch("march_kernel");
 }

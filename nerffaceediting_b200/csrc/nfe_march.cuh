@@ -6,7 +6,6 @@ namespace nfe {
 
 constexpr int MARCH_SMEM_FLOATS_PER_SAMPLE = 5;  // depth, sigma, weight, order, unsorted sigma
 constexpr int MARCH_GROUP_PAIRS = 2;  // row pairs per ring group (one cp.async per lane and pair); 2 halves the wait/commit/loop overhead per row: same box, 0.138 -> 0.125 ms
-constexpr int MARCH_RING_GROUP_BYTES = MARCH_GROUP_PAIRS * 2 * 192;  // one ring group = pairs of 192-byte record rows (one row per half-warp)
 constexpr int MAX_S = 768;  // merged samples per ray (reference configs go up to 192+192, SURVEY.md §8a)
 
 struct MarchArgs {
@@ -14,7 +13,7 @@ struct MarchArgs {
     const float* depths1; const float* colors1; const float* segs1; const float* sigma1; int s1;
     const float* depths2; const float* colors2; const float* segs2; const float* sigma2; int s2;
     // packed alternative to colors/segs (the fused render's workspace): rec[row] = {sigma, seg[15], rgb[32]}, 48 floats;
-    // implies cc = 32 and cs = 15 or 0
+    // implies cc = 32 and cs = 15 or 0 — or, with cc = 0 and cs = 15 (a geometry-only render), rec[row] = {sigma, seg[15]}, 16 floats
     const float* rec1; const float* rec2;
     int64_t n_rays;
     int cc, cs;        // colour / semantic channels (0: weights only)

@@ -12,6 +12,7 @@ namespace {
 struct Workspace {
     float* minmax;    // 2 floats (+pad)
     float* sigma_c; float* rec_c;   // densities (compact, for the weights / merge) and packed records {sigma,seg[15],rgb[32]}
+                                    // ({sigma,seg[15]} in a geometry-only render, none for its OSG decoder: see record_floats)
     float* w_c;       // [T, s_c-1], not written: resample_kernel forms the coarse weights itself.  Its size stays in
                       // nfe_render_workspace_bytes, which sets how ops.render_fwd chunks a large render (and so each chunk's Philox offset)
     float* depths_f;  // [T, s_f]
@@ -20,6 +21,14 @@ struct Workspace {
 };
 
 int64_t align256(int64_t x) { return (x + 255) / 256 * 256; }
+
+// floats per sample record: {sigma, seg[15], rgb[32]}; a geometry-only render keeps {sigma, seg[15]}, and its OSG decoder
+// (no semantics) only the densities
+int64_t record_floats(const nfe_render_cfg* cfg)
+{
+    if (!cfg->geometry_only) return 48;
+    return cfg->kind == NFE_DEC_OSG ? 0 : 16;
+}
 
 Workspace carve(const nfe_render_cfg* cfg, int64_t rays, void* base)
 {
@@ -31,15 +40,15 @@ Workspace carve(const nfe_render_cfg* cfg, int64_t rays, void* base)
         off += align256(floats * (int64_t)sizeof(float));
         return r;
     };
-    const int64_t sc = cfg->s_c, sf = cfg->s_f;
+    const int64_t sc = cfg->s_c, sf = cfg->s_f, rec = record_floats(cfg);
     w.minmax = take(64);
     w.sigma_c = take(rays * sc);
-    w.rec_c = take(rays * sc * 48);
+    w.rec_c = take(rays * sc * rec);
     if (sf > 0) {
         w.w_c = take(rays * (sc - 1));
         w.depths_f = take(rays * sf);
         w.sigma_f = take(rays * sf);
-        w.rec_f = take(rays * sf * 48);
+        w.rec_f = take(rays * sf * rec);
     }
     w.bytes = off;
     return w;
@@ -56,6 +65,7 @@ NFE_EXPORT int64_t nfe_render_workspace_bytes(const nfe_render_cfg* cfg, int n, 
 NFE_EXPORT int nfe_render_workspace_layout(const nfe_render_cfg* cfg, int n, int64_t n_rays, int64_t* offsets)
 {
     NFE_REQUIRE(cfg && offsets && n >= 0 && n_rays >= 0, "nfe_render_workspace_layout: bad arguments");
+    NFE_REQUIRE(!cfg->geometry_only, "nfe_render_workspace_layout: a geometry_only render has no backward and no workspace layout for it");
     const Workspace w = carve(cfg, (int64_t)n * n_rays, nullptr);
     auto off = [](const float* p) { return p ? (int64_t)(reinterpret_cast<const char*>(p) - static_cast<const char*>(nullptr)) : (int64_t)-1; };
     offsets[0] = off(w.sigma_c); offsets[1] = off(w.rec_c); offsets[2] = cfg->s_f > 0 ? off(w.sigma_f) : -1; offsets[3] = cfg->s_f > 0 ? off(w.rec_f) : -1;
@@ -79,21 +89,23 @@ NFE_EXPORT int nfe_render_fwd(const nfe_render_cfg* cfg, const nfe_mlp* net_a, c
     if (rays == 0) return 0;  // empty tensors carry null pointers
     const int sc = cfg->s_c, sf = cfg->s_f;
     const int64_t pass_samples = n_rays * (sf > 0 && sf < sc ? sf : sc);
+    const bool geometry = cfg->geometry_only != 0;
     FieldArgs f = {};
-    if (int rc = field_planes(cfg, planes_norm_cl, planes_denorm_cl, plane_batch, n, pass_samples, false, "nfe_render_fwd", f)) return rc;
-    NFE_REQUIRE(origins && dirs && depths_coarse && rgb && depth && wsum, "nfe_render_fwd: null pointer");
+    if (int rc = field_planes(cfg, planes_norm_cl, planes_denorm_cl, plane_batch, n, pass_samples, false, geometry, "nfe_render_fwd", f)) return rc;
+    NFE_REQUIRE(origins && dirs && depths_coarse && (rgb || geometry) && depth && wsum, "nfe_render_fwd: null pointer");
     NFE_REQUIRE(cfg->seg_dim == 0 || seg, "nfe_render_fwd: seg output missing");
     NFE_REQUIRE(cfg->s_f == 0 || cfg->stochastic || u_fine, "nfe_render_fwd: parity mode needs the u_fine table");
     NFE_REQUIRE(workspace, "nfe_render_fwd: null workspace");
     const Workspace w = carve(cfg, rays, workspace);
     NFE_REQUIRE(workspace_bytes >= w.bytes, "nfe_render_fwd: workspace too small (%lld < %lld bytes)", (long long)workspace_bytes, (long long)w.bytes);
+    const bool records = record_floats(cfg) > 0;   // the OSG decoder's geometry-only passes write densities alone
     cudaStream_t stream = as_stream(stream_);
     float* minmax = minmax_out ? minmax_out : w.minmax;
 
     // ---- coarse pass (renderer.py:104-113,325-336)
     f.origins = origins; f.dirs = dirs; f.depths = depths_coarse; f.s_per_ray = sc;
     f.m = n_rays * sc; f.total = rays * sc;
-    f.sigma = w.sigma_c; f.rec = w.rec_c;
+    f.sigma = w.sigma_c; f.rec = records ? w.rec_c : nullptr;
     f.density_noise = cfg->density_noise; f.seed = cfg->seed; f.offset = cfg->offset + 1;
     {
         StageScope t(STAGE_FIELD_COARSE, stream);
@@ -117,17 +129,18 @@ NFE_EXPORT int nfe_render_fwd(const nfe_render_cfg* cfg, const nfe_mlp* net_a, c
         }
         // ---- fine pass (renderer.py:122-129,344-353)
         f.depths = df; f.s_per_ray = sf; f.m = n_rays * sf; f.total = rays * sf;
-        f.sigma = w.sigma_f; f.rec = w.rec_f; f.offset = cfg->offset + 3;
+        f.sigma = w.sigma_f; f.rec = records ? w.rec_f : nullptr; f.offset = cfg->offset + 3;
         {
             StageScope t(STAGE_FIELD_FINE, stream);
             if (int rc = launch_field(cfg->kind, cfg->precision, f, net_a, net_b, stream)) return rc;
         }
         // ---- merge + composite (renderer.py:131-135,355-359)
-        m.depths2 = df; m.rec2 = w.rec_f; m.sigma2 = w.sigma_f; m.s2 = sf;
+        m.depths2 = df; m.rec2 = records ? w.rec_f : nullptr; m.sigma2 = w.sigma_f; m.s2 = sf;
         m.inputs_sorted = 1;  // coarse depths ascend by construction; the fine list is emitted sorted (table u, or sort_u)
     }
-    m.depths1 = depths_coarse; m.rec1 = w.rec_c; m.sigma1 = w.sigma_c; m.s1 = sc;
-    m.cc = 32; m.cs = cfg->seg_dim; m.rgb = rgb; m.seg = seg; m.depth = depth; m.wsum = wsum; m.weights = nullptr; m.minmax = minmax;
+    m.depths1 = depths_coarse; m.rec1 = records ? w.rec_c : nullptr; m.sigma1 = w.sigma_c; m.s1 = sc;
+    // geometry-only: no colour channels (records {sigma, seg[15]}, or for OSG the weights alone: depth and wsum)
+    m.cc = geometry ? 0 : 32; m.cs = cfg->seg_dim; m.rgb = geometry ? nullptr : rgb; m.seg = seg; m.depth = depth; m.wsum = wsum; m.weights = nullptr; m.minmax = minmax;
     m.image_rays = cfg->image_layout ? n_rays : 0;
     StageScope t(STAGE_MARCH_FINAL, stream);
     if (int rc = launch_march(m, sf > 0, stream)) return rc;

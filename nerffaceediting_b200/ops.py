@@ -476,7 +476,8 @@ def workspace_limit_bytes():
 
 def render_fwd(cfg, seq_a, seq_b, planes_norm_cl, planes_denorm_cl, origins, dirs, depths_coarse, u_fine,
                finish_depth=True, return_stages=False, keep_workspace=False):
-    """Fused forward.  Returns (rgb [N,R,32], seg [N,R,15]|None, depth [N,R,1], wsum [N,R,1], minmax [2][, stages]).
+    """Fused forward.  Returns (rgb [N,R,32], seg [N,R,15]|None, depth [N,R,1], wsum [N,R,1], minmax [2][, stages]); rgb is None
+    when cfg.geometry_only is set.
     keep_workspace (training): the stages dict also carries views of the per-sample densities / records the
     backward re-reads (sigma_c, rec_c, sigma_f, rec_f) and keeps the workspace alive."""
     o, d = _cuda_f32(origins, "ray_origins"), _cuda_f32(dirs, "ray_directions")
@@ -488,7 +489,7 @@ def render_fwd(cfg, seq_a, seq_b, planes_norm_cl, planes_denorm_cl, origins, dir
     a = MlpRef(seq_a, dev)
     b = MlpRef(seq_b, dev) if seq_b is not None else None
     image = bool(cfg.image_layout)
-    rgb = torch.empty((n, 32, r) if image else (n, r, 32), device=dev, dtype=torch.float32)
+    rgb = None if cfg.geometry_only else torch.empty((n, 32, r) if image else (n, r, 32), device=dev, dtype=torch.float32)
     seg = torch.empty((n, cfg.seg_dim, r) if image else (n, r, cfg.seg_dim), device=dev, dtype=torch.float32) if cfg.seg_dim else None
     depth = torch.empty((n, r, 1), device=dev, dtype=torch.float32)
     wsum = torch.empty((n, r, 1), device=dev, dtype=torch.float32)
@@ -526,7 +527,7 @@ def render_fwd(cfg, seq_a, seq_b, planes_norm_cl, planes_denorm_cl, origins, dir
         if image and cr != r:
             raise RuntimeError("render_fwd: image-layout outputs cannot be split into ray blocks; raise NFE_WORKSPACE_MB")
         map_sl = (slice(i0, i1),) if image else sl            # image layout [n, C, r]: only whole items can be sliced
-        views = [rgb[map_sl], None if seg is None else seg[map_sl], depth[sl], wsum[sl]]
+        views = [None if rgb is None else rgb[map_sl], None if seg is None else seg[map_sl], depth[sl], wsum[sl]]
         direct = all(v is None or v.is_contiguous() for v in views)
         bufs = views if direct else [None if v is None else torch.empty_like(v) for v in views]
         rc = lib.nfe_render_fwd(ctypes.byref(ccfg), a.ref(), b.ref() if b else None, _ptr(pn), _ptr(pd), (pn if pd is None else pd).shape[0], _ptr(oo), _ptr(dd), cn, cr,
@@ -540,7 +541,13 @@ def render_fwd(cfg, seq_a, seq_b, planes_norm_cl, planes_denorm_cl, origins, dir
 
     with _Guard(o):
         limit = workspace_limit_bytes()
-        per_item = lib.nfe_render_workspace_bytes(ctypes.byref(cfg), 1, r) if n and r else 0
+        plan_cfg = cfg
+        if cfg.geometry_only and (cfg.stochastic or cfg.density_noise > 0):
+            # every chunk draws its jitter and density noise from its own Philox offset: a geometry-only render whose draws
+            # must match the full render's splits where the full render would, and allocates only its smaller workspace
+            plan_cfg = NfeRenderCfg.from_buffer_copy(cfg)
+            plan_cfg.geometry_only = 0
+        per_item = lib.nfe_render_workspace_bytes(ctypes.byref(plan_cfg), 1, r) if n and r else 0
         if n * per_item <= limit or n * r == 0 or keep_workspace:
             call(0, n, 0, r, minmax, finish_depth)
         else:

@@ -24,6 +24,12 @@ Extra keys read from `rendering_options` (all optional; defaults reproduce the r
                             what triplane.py:122-125 builds with three permute+reshape+contiguous passes — written in that
                             layout by the compositing kernel itself.
   nfe_cache_planes   False  keep the channel-last staging of the planes between calls (video sweeps).
+  nfe_geometry_only  False  render geometry alone: forward returns (None, seg, depth, wsum) (disentangled) or (None, depth, wsum),
+                            bit-identical to the full render's maps, without the appearance branch: no colours are decoded or
+                            composited, the per-sample records shrink to a third, and the disentangled decoder reads only the
+                            normalised planes (the raw ones are neither staged nor gathered); a render with draws is split into
+                            workspace chunks where the full render would be, so it draws the same samples.  Inference only; the staged path
+                            (other decoders) honours the same outputs but saves nothing.
 
 Instances hold no state of their own beyond the reference's attributes, so objects unpickled from
 reference checkpoints (which skip __init__, SURVEY.md §7.9) work.
@@ -45,6 +51,7 @@ class FieldPlan(NamedTuple):
     seq_b: object           # None for the OSG decoder
     precision: int
     geo_only: bool          # density-only query, disentangled decoder on the tensor cores: the appearance net and its planes are skipped
+    geometry: bool          # geometry-only render (rendering_options['nfe_geometry_only']): no colours; disentangled: geo_net on the normalised planes
     affine: object          # (scale [K,96], shift [K,96]) under the single-gather identity, else None
     sources: object         # training under the identity: (scale_src, shift_src), the autograd inputs of the affine pair, else None
     stage_norm: bool        # which plane sets are staged channel-last
@@ -53,14 +60,18 @@ class FieldPlan(NamedTuple):
     path: object            # (what, path) for ops.note_path, or None
 
 
-def field_plan(what, desc, norm_planes, planes, opts, batch, per_item, grad, sigma_only=False):
+def field_plan(what, desc, norm_planes, planes, opts, batch, per_item, grad, sigma_only=False, geometry=False):
     """Decide the fused forward of one call: what = 'render' (per_item rays per batch item) or 'run_model' (per_item points),
-    desc = ops.describe_decoder(decoder), grad = whether the call is differentiable.  It reads the options, the environment
-    and the plane registries and calls no kernel, so it runs on CPU tensors as well."""
+    desc = ops.describe_decoder(decoder), grad = whether the call is differentiable, geometry = a geometry-only render
+    (inference only).  It reads the options, the environment and the plane registries and calls no kernel, so it runs on CPU
+    tensors as well."""
     kind, seq_a, seq_b = desc
     precision = ops.precision_of(opts)
     disentangled_tc = kind == ops.DEC_DISENTANGLED and precision != ops.PRECISIONS['fp32']
     geo_only = sigma_only and disentangled_tc
+    # geometry-only render, disentangled decoder: geo_net reads the normalised planes alone (every precision), so the raw
+    # planes are neither staged nor gathered and their provenance is not needed
+    norm_only = geometry and kind == ops.DEC_DISENTANGLED
     library_gemm = os.environ.get("NFE_BWD_LIBRARY_GEMM", "0") == "1"
     if what == "render":
         s_c, s_f = opts['depth_resolution'], opts['depth_resolution_importance']
@@ -73,9 +84,11 @@ def field_plan(what, desc, norm_planes, planes, opts, batch, per_item, grad, sig
     if not grad:
         # planes known to be norm*scale + shift per channel (normalize_plane / denormalize_plane made them): gather the
         # normalised planes only and rebuild the de-normalised features from the statistics
-        if single and not geo_only:
+        if single and not geo_only and not norm_only:
             affine = ops.provenance(norm_planes, planes)
         path = (what, "single-gather" if (affine is not None or geo_only) else ("two-gather" if kind == ops.DEC_DISENTANGLED else "one-set"))
+        if geometry:
+            path = (what, "geometry-only")
     else:
         # In training the identity replaces the gradient into `planes` by gradients into the normalised planes and the
         # statistics `planes` is tied to (normalize_plane: planes is their root; denormalize_plane: planes is their product),
@@ -92,8 +105,8 @@ def field_plan(what, desc, norm_planes, planes, opts, batch, per_item, grad, sig
             sources = (scale_src, shift_src)
         path = (what, "training-single-gather" if sources else "training") if what == "render" else None
     # a differentiable run_model stages the raw planes even when geometry-only: its backward returns their gradient in that shape
-    return FieldPlan(kind, seq_a, seq_b, precision, geo_only, affine, sources, kind == ops.DEC_DISENTANGLED,
-                     affine is None and not (geo_only and not grad), library_gemm, path)
+    return FieldPlan(kind, seq_a, seq_b, precision, geo_only, geometry, affine, sources, kind == ops.DEC_DISENTANGLED,
+                     affine is None and not (geo_only and not grad) and not norm_only, library_gemm, path)
 
 
 def _stage(plan, norm_planes, planes, cache):
@@ -115,6 +128,7 @@ def render_planes(plan, norm_planes, planes, origins, dirs, depths_coarse, u_fin
                        opts.get('white_back', False), opts.get('density_noise', 0) or 0.0, stochastic=stochastic, seed=seed, offset=offset,
                        precision=plan.precision, affine=plan.affine)
     cfg.image_layout = int(image_layout)
+    cfg.geometry_only = int(plan.geometry)
     return cfg, norm_cl, denorm_cl, ops.render_fwd(cfg, plan.seq_a, plan.seq_b, norm_cl, denorm_cl, origins, dirs, depths_coarse, u_fine, **taps)
 
 
@@ -238,17 +252,26 @@ class ImportanceRenderer(torch.nn.Module):
             # silently detaching would be wrong
             raise RuntimeError("ImportanceRenderer: gradients w.r.t. ray_origins / ray_directions are not built; detach the rays")
         deterministic = bool(opts.get('nfe_deterministic', False))
+        geometry = bool(opts.get('nfe_geometry_only', False))
+        if geometry:
+            if defer_clamp:
+                raise NotImplementedError("rendering_options['nfe_geometry_only'] is not built for the ray-sharded render")
+            params = tuple(decoder.parameters()) if isinstance(decoder, nn.Module) else ()
+            if torch.is_grad_enabled() and any(isinstance(t, torch.Tensor) and t.requires_grad for t in (norm_planes, planes, *params)):
+                raise RuntimeError("rendering_options['nfe_geometry_only'] is inference-only (it has no backward): "
+                                   "call under torch.no_grad() or detach the inputs")
         desc = self._fused_decoder(decoder, norm_planes)
         if desc is None:
             ops.note_path("render", "staged")
             if defer_clamp:
                 raise NotImplementedError("a ray-sharded render needs one of the reference's decoders (fused path)")
-            return self._render_staged(norm_planes, planes, decoder, ray_origins, ray_directions, opts, deterministic)
+            rgb, seg, depth, wsum = self._render_staged(norm_planes, planes, decoder, ray_origins, ray_directions, opts, deterministic)
+            return (None if geometry else rgb), seg, depth, wsum      # geometry-only: the caller's decoder ran in full, rgb is dropped
         grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (norm_planes, planes, *decoder.parameters()))
         if grad and defer_clamp:
             raise NotImplementedError("the ray-sharded render is inference-only")
         n, r, _ = ray_origins.shape
-        plan = field_plan("render", desc, norm_planes, planes, opts, n, r, grad)
+        plan = field_plan("render", desc, norm_planes, planes, opts, n, r, grad, geometry=geometry)
         ops.note_path(*plan.path)
         image = bool(opts.get('nfe_image_layout', False)) and not defer_clamp and not grad
         side = int(round(r ** 0.5))
@@ -272,7 +295,7 @@ class ImportanceRenderer(torch.nn.Module):
         if defer_clamp:
             return rgb, seg, depth, wsum, minmax
         if image:
-            return (rgb.view(n, 32, side, side), None if seg is None else seg.view(n, seg.shape[1], side, side),
+            return (None if rgb is None else rgb.view(n, 32, side, side), None if seg is None else seg.view(n, seg.shape[1], side, side),
                     depth.view(n, 1, side, side), wsum)
         return rgb, seg, depth, wsum
 

@@ -103,6 +103,7 @@ class ShardedRenderer:
         self.last_packed = None          # this rank's packed [rgb|seg|depth|wsum] maps of the latest local_batch call
 
     def __call__(self, norm_planes, planes, decoder, ray_origins, ray_directions, rendering_options, local_batch=False):
+        _no_geometry_only(rendering_options)
         world = dist.get_world_size(self.group) if (dist.is_available() and dist.is_initialized()) else 1
         if not local_batch or world == 1:
             out = render_sharded(self.renderer, norm_planes, planes, decoder, ray_origins, ray_directions, rendering_options, group=self.group)
@@ -152,6 +153,11 @@ class ShardedRenderer:
             torch.cuda.current_stream().wait_stream(self._stream)
 
 
+def _no_geometry_only(rendering_options):
+    if rendering_options.get('nfe_geometry_only', False):
+        raise NotImplementedError("rendering_options['nfe_geometry_only'] is not built for the sharded renderer")
+
+
 def render_sharded(renderer, norm_planes, planes, decoder, ray_origins, ray_directions, rendering_options, group=None,
                    render_local=None, finish=None, force_sharded_path=False):
     """Sharded forward of ImportanceRenderer (norm_planes=None) / DisentangledImportanceRenderer.
@@ -159,6 +165,7 @@ def render_sharded(renderer, norm_planes, planes, decoder, ray_origins, ray_dire
     `render_local` / `finish` are injection points for tests; by default they call the renderer's deferred-clamp
     entry and nfe_finish_depth.  force_sharded_path=True takes the sharded code path (deferred clamp, range reduction,
     pack / pad / all-gather / unpack) even in a world of one — what a single-GPU box can test of it."""
+    _no_geometry_only(rendering_options)
     initialized = dist.is_available() and dist.is_initialized()
     if (not initialized or dist.get_world_size(group) == 1) and not (force_sharded_path and initialized):
         return renderer._render(norm_planes, planes, decoder, ray_origins, ray_directions, rendering_options)
